@@ -11,9 +11,11 @@ semantics).  `value` is measured with the packed syndromes already resident in H
 the C-ABI host-buffer call (host BitMatrix in, BitMatrix + success out, copies inside the timed
 region; `e2e_by_format` adds pageable buffers and the Matrix{Int} input of the reference's own test).
 Under torchrun every rank decodes its own 10M-syndrome shard (weak scaling, inputs keyed by the
-global syndrome index) and the counters are all-reduced over NCCL.  At N = 1 the line also carries
-short sub-records of the other BASELINE configs at their full batch sizes (C2 per sweep, C4 10M tiled,
-C5 1M streamed).
+global syndrome index) and the counters are all-reduced over NCCL.  At N = 1 a second JSON line, on
+stderr, carries extra operating points and short sub-records of the other BASELINE configs at their
+full batch sizes (C2 per sweep, C4 10M tiled, C5 1M streamed).
+
+  python bench.py --dump-outputs DIR ...    # also write what the last timed step computed to DIR/*.npy
 """
 import argparse
 import glob
@@ -124,8 +126,8 @@ def measured_peaks():
 
 
 def ncu_record(workload, variant, kernel_rev):
-    """The tracked ncu summary (profiles/*.json, written by tools/ncu_summary.py --json on the GPU box) of this
-    workload's dominant kernel, newest round first.  None if no capture is committed -- never a literal."""
+    """The tracked ncu summary (profiles/*.json, written by tools/ncu_summary.py --json) of this workload's dominant
+    kernel, newest round first.  None if no capture is committed -- never a literal.  Records name it by its "file"."""
     for path in sorted(glob.glob(os.path.join(ROOT, "profiles", "r*_ncu_*.json")), reverse=True):
         try:
             d = json.load(open(path))
@@ -221,7 +223,17 @@ def protect_stdout():
         os.dup2(2, 1)
 
 
+# Extra operating points and the other configs' sub-records: a second JSON line on stderr, so that the result line keeps
+# to the headline and stays a few KB (tools that read a command's output tail cannot parse a line of tens of KB).
+DETAIL_KEYS = ("e2e_by_format", "sweep", "minsum", "fast32", "bposd_osd0", "config_C2_surface_d15_1M", "config_C4_hgp1600_10M",
+               "config_C5_gallager100k_1M")
+
+
 def emit(line):
+    detail = {k: line.pop(k) for k in DETAIL_KEYS if k in line}
+    if detail:
+        sys.stderr.write(json.dumps({"detail": detail}) + "\n")
+        sys.stderr.flush()
     out = _REAL_STDOUT if _REAL_STDOUT is not None else sys.stdout
     out.write(json.dumps(line) + "\n")
     out.flush()
@@ -295,6 +307,29 @@ class DeviceRun:
         self.kernel_s, self.kernel_launches = kms / 1e3, kl       # summed over the timed steps
         return secs, total.cpu().numpy(), self.dec.launch_count() - l0
 
+    def dump_last_step(self, out_dir, n, max_bytes=56 << 20):
+        """What the last timed step returned to its caller, as .npy files in out_dir: for a fixed, seeded sample of the
+        syndromes of the last tile decoded, their global indices, decoded errors (one row per syndrome), converged flags
+        and iteration counts, plus the whole step's counters (decoded, converged, iterations).  The sample keeps the
+        files under max_bytes."""
+        torch = self.torch
+        t0 = (self.B - 1) // self.tile * self.tile
+        bt = self.B - t0
+        k = int(min(bt, 65536, max(1, max_bytes // (4 * (n + 2) + 8))))
+        local = np.sort(np.random.default_rng(SEED_E).choice(bt, size=k, replace=False))
+        idx = torch.from_numpy(local).to(self.dev)
+        torch.cuda.synchronize()
+        words = self.errw[idx].cpu().numpy().view(np.uint8)            # bit r % 32 of little-endian word r / 32
+        errors = np.unpackbits(words, axis=1, bitorder="little")[:, :n]
+        os.makedirs(out_dir, exist_ok=True)
+        out = {"syndrome_index": (self.first + t0 + local).astype(np.float64),
+               "errors": errors.astype(np.float32),
+               "converged": self.conv[idx].cpu().numpy().astype(np.float32),
+               "iterations": self.iters[idx].cpu().numpy().astype(np.float32),
+               "counters": self.ctr[:3].cpu().numpy().astype(np.float64)}
+        for name, a in out.items():
+            np.save(os.path.join(out_dir, name + ".npy"), a)
+
     def exact_match_frac_last_tile(self, per):
         """Exact-match fraction of the LAST tile decoded (its true errors are regenerated from the same stream)."""
         torch = self.torch
@@ -343,7 +378,7 @@ def roofline_of(info, variant, E, SW, NW, B_per_step_gpu, units_per_step_gpu, st
                         "figure, not a pipe utilisation); peak = %d SMs x 64 FP64 lanes/clk x median SM clock under load (%.0f MHz); one FLOP = "
                         "one FP64 lane-instruction" % (
                             slots["model"], "reference" if variant == "exact" else variant, slots["executed"], info["sm_count"], clk_mhz),
-                "ncu": ncu,
+                "ncu": ncu and ncu["file"],
                 "hbm_model": {"achieved_GBps": alg_bytes / step_s / 1e9, "peak_GBps": peaks["hbm_gbs"], "peak_source": peaks_src,
                               "frac": alg_bytes / step_s / 1e9 / peaks["hbm_gbs"],
                               "note": "4*E*8 B per syndrome-iteration if messages lived in HBM (they live in shared memory) + packed I/O"}}
@@ -357,7 +392,7 @@ def roofline_of(info, variant, E, SW, NW, B_per_step_gpu, units_per_step_gpu, st
                 "note": "algorithmic bytes = 4*E*8 per syndrome-iteration + packed I/O of the kernel's launches / the kernel's own CUDA-event time; "
                         "peak = %s copy bandwidth; message store %d MB per GPU; traffic = ncu dram bytes of one profiled launch scaled to this "
                         "run's launch size" % (peaks_src, info["message_bytes"] >> 20),
-                "ncu": ncu}
+                "ncu": ncu and ncu["file"]}
     return roof
 
 
@@ -451,7 +486,12 @@ def main():
                     help="extra ldpcb200_set_option pairs (experiments), e.g. --opt dual=1")
     ap.add_argument("--variant", default="exact", choices=["exact", "minsum", "fast"],
                     help="exact = reference-parity sum-product (headline); minsum = normalised min-sum (no reference equivalent)")
+    ap.add_argument("--dump-outputs", default=None, dest="dump_outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (a seeded sample of "
+                         "the decoded syndromes, at most 64 MB), so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.single_process):
+        ap.error("--dump-outputs applies to the device-resident run (--impl ours without --single-process)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -526,6 +566,8 @@ def main():
     sampler.start()                               # clocks are sampled during the timed region only
     secs, c, launches = run.timed(args.steps, 0, flush, allreduce, barrier)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        run.dump_last_step(args.dump_outputs, n)
     t = torch.tensor([secs], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
