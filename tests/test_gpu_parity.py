@@ -1098,8 +1098,16 @@ def test_first_iteration_filter_properties(pkg, oracle, codes):
         for a, b in zip(outs[0], outs[1]):
             assert np.array_equal(a, b), variant
         assert (outs[0][2] == 1).mean() > 0.8 and outs[0][3][0] == B and outs[0][3][2] == int(outs[0][2].sum())
-    ref = oracle.batch_decode(H, 0.01, 32, syn[:, :20000], nthreads=oracle.num_threads())
-    assert np.array_equal(outs[0][0][:, :20000], oracle.batch_decode(H, 0.01, 32, syn[:, :20000], nthreads=oracle.num_threads(), variant="fast")["errors"]) or True
+    # the filtered fast-variant outputs (the last variant above, filter on) against the variant's CPU definition, with the
+    # statistical bar of test_fast32_variant_tracks_its_definition
+    syn_f = syn[:, :20000]
+    ref_f = oracle.batch_decode(H, 0.01, 32, syn_f, nthreads=oracle.num_threads(), variant="fast")
+    err_f, conv_f, it_f = outs[0][0][:, :20000], outs[0][1][:20000], outs[0][2][:20000]
+    assert ((err_f != ref_f["errors"]).any(axis=0) | (conv_f != ref_f["converged"])).mean() <= 0.02
+    assert abs(conv_f.mean() - ref_f["converged"].mean()) <= 0.005
+    assert abs(it_f.mean() - ref_f["iters"].mean()) <= 0.02 * ref_f["iters"].mean() + 0.01
+    assert (((H @ err_f) % 2 == syn_f).all(axis=0) == conv_f).all()
+    ref = oracle.batch_decode(H, 0.01, 32, syn_f, nthreads=oracle.num_threads())
     dec = pkg.BeliefPropagationDecoder(H, 0.01, 32)
     errors = np.zeros((144, 20000), dtype=np.uint8, order="F")
     iters = np.zeros(20000, dtype=np.int32)
