@@ -83,11 +83,11 @@ def brute_force_ratio(H, per, syndrome):
         return p1 / p0
 
 
-def osd0_dense(H, syndrome, bp_err, ratio):
+def osd0_dense(H, syndrome, bp_err, ratio, return_pivots=False):
     """Dense transliteration of decode!(::BeliefPropagationOSDDecoder) after the BP call
     (belief_propagation_osd.jl:52-60) and of osd(..., Val(0)) (:63-125), numpy bool matrices, physical
     row swaps, same loop order.  r = 1/R replaces exp(log(1/R)) exactly as in bp_oracle.c.
-    Also the mathematical characterisation used to double check it: see osd0_by_definition."""
+    With return_pivots: (result, number of pivots used)."""
     H = np.asarray(H).astype(bool)
     m, n = H.shape
     with np.errstate(all="ignore"):
@@ -100,6 +100,7 @@ def osd0_dense(H, syndrome, bp_err, ratio):
     for j in range(n):
         if e[j] == 1:
             t ^= Hs[:, j]
+    rows, cols = [], []
     if not t.any():
         corr = e.astype(bool)
     else:
@@ -134,7 +135,7 @@ def osd0_dense(H, syndrome, bp_err, ratio):
                         t[ii] ^= True
     out = np.zeros(n, dtype=np.uint8)
     out[np.asarray(order)] = corr.astype(np.uint8)
-    return out
+    return (out, len(rows)) if return_pivots else out
 
 
 def osdk_dense(H, syndrome, bp_err, ratio, osd_order):

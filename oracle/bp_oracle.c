@@ -768,3 +768,45 @@ int bp_oracle_bposd_batch(int64_t s, int64_t n, const int64_t *colptr, const int
     free_graph(&g);
     return fail ? -1 : 0;
 }
+
+/* OSD-0 (osd0_one) on caller-supplied BP decisions and posterior ratios, every column: osd(..., Val(0)) as a function of
+ * (syndrome, bp_err, ratio) alone, whatever produced them.  syn: s x B, bp_err: n x B bytes, ratio: n x B doubles, all
+ * column-major; err_out: n x B bytes, pivots_out: optional B int32 (pivots used; 0 where bp_err already satisfies the
+ * syndrome). */
+int bp_oracle_osd0_given(int64_t s, int64_t n, const int64_t *colptr, const int64_t *rowval, int64_t B, const uint8_t *syn,
+                         const uint8_t *bp_err, const double *ratio, uint8_t *err_out, int32_t *pivots_out, int32_t nthreads)
+{
+    graph_t g;
+    int rc = build_graph(&g, s, n, colptr, rowval);
+    if (rc) return rc;
+    if (nthreads < 1) nthreads = 1;
+    int fail = 0;
+    const size_t nn = (size_t)(n ? n : 1), ss = (size_t)(s ? s : 1), nw = (size_t)((n + 63) / 64 + 1);
+#ifdef _OPENMP
+#pragma omp parallel num_threads(nthreads)
+#endif
+    {
+        uint8_t *tgt = (uint8_t *)malloc(ss), *es = (uint8_t *)malloc(nn), *corr = (uint8_t *)malloc(nn);
+        keyidx_t *ki = (keyidx_t *)malloc(sizeof(keyidx_t) * nn);
+        uint64_t *Hw = (uint64_t *)malloc(sizeof(uint64_t) * ss * nw);
+        int64_t *pr = (int64_t *)malloc(sizeof(int64_t) * ss), *pc = (int64_t *)malloc(sizeof(int64_t) * ss);
+        if (!tgt || !es || !corr || !ki || !Hw || !pr || !pc) {
+#ifdef _OPENMP
+#pragma omp atomic write
+#endif
+            fail = 1;
+        } else {
+#ifdef _OPENMP
+#pragma omp for schedule(dynamic, 4)
+#endif
+            for (int64_t c = 0; c < B; ++c) {
+                const int np = osd0_one(&g, colptr, rowval, syn + (size_t)c * (size_t)s, bp_err + (size_t)c * (size_t)n,
+                                        ratio + (size_t)c * (size_t)n, err_out + (size_t)c * (size_t)n, ki, Hw, tgt, es, corr, pr, pc);
+                if (pivots_out) pivots_out[c] = np;
+            }
+        }
+        free(tgt); free(es); free(corr); free(ki); free(Hw); free(pr); free(pc);
+    }
+    free_graph(&g);
+    return fail ? -1 : 0;
+}

@@ -53,6 +53,9 @@ def load():
     lib.bp_oracle_bposd_order_batch.restype = ctypes.c_int
     lib.bp_oracle_bposd_order_batch.argtypes = [ctypes.c_int64, ctypes.c_int64, i64p, i64p, ctypes.c_double, ctypes.c_int32, ctypes.c_int32,
                                                 ctypes.c_int64, u8p, u8p, u8p, ctypes.c_int32]
+    lib.bp_oracle_osd0_given.restype = ctypes.c_int
+    lib.bp_oracle_osd0_given.argtypes = [ctypes.c_int64, ctypes.c_int64, i64p, i64p, ctypes.c_int64, u8p, u8p,
+                                         ctypes.POINTER(ctypes.c_double), u8p, ctypes.POINTER(ctypes.c_int32), ctypes.c_int32]
     lib.bpots_oracle_batch.restype = ctypes.c_int
     lib.bpots_oracle_batch.argtypes = [ctypes.c_int64, ctypes.c_int64, i64p, i64p, ctypes.c_double, ctypes.c_int32, ctypes.c_int32,
                                        ctypes.c_double, ctypes.c_int64, u8p, u8p, u8p, ctypes.POINTER(ctypes.c_int32), ctypes.c_int32]
@@ -138,6 +141,31 @@ def bposd_decode(H, per, max_iters, syndromes, nthreads=1, key_mode=0):
     if rc != 0:
         raise RuntimeError("bp_oracle_bposd_batch failed: %d" % rc)
     return dict(errors=err, converged=conv.astype(bool), bp_errors=bp, pivots=piv)
+
+
+def osd0_given(H, syndromes, bp_err, ratio, nthreads=1):
+    """osd(..., Val(0)) behind the reliability sort (belief_propagation_osd.jl:52-60, :63-125) on caller-supplied BP
+    decisions bp_err (n,B) and posterior ratios ratio (n,B), every column -- no BP call, and no shortcut for columns BP
+    would call converged (bp_err satisfying the syndrome comes back unchanged with 0 pivots).  Returns dict(errors (n,B)
+    uint8, pivots (B,) int32)."""
+    lib = load()
+    lib.bp_oracle_set_osd_key_mode(0)                 # the kernel's key, RN(1/R)
+    s, n, colptr, rowval = csc_arrays(H)
+    syn = np.asfortranarray(np.asarray(syndromes).astype(np.uint8))
+    if syn.ndim == 1:
+        syn = np.asfortranarray(syn.reshape(s, 1))
+    B = syn.shape[1]
+    e =np.asfortranarray(np.asarray(bp_err).astype(np.uint8).reshape(n, B))
+    r = np.asfortranarray(np.asarray(ratio, dtype=np.float64).reshape(n, B))
+    assert syn.shape[0] == s
+    err = np.zeros((n, B), dtype=np.uint8, order="F")
+    piv = np.zeros(B, dtype=np.int32)
+    rc = lib.bp_oracle_osd0_given(s, n, _p(colptr, ctypes.c_int64), _p(rowval, ctypes.c_int64), B, _p(syn, ctypes.c_uint8),
+                                  _p(e, ctypes.c_uint8), _p(r, ctypes.c_double), _p(err, ctypes.c_uint8),
+                                  _p(piv, ctypes.c_int32), int(nthreads))
+    if rc != 0:
+        raise RuntimeError("bp_oracle_osd0_given failed: %d" % rc)
+    return dict(errors=err, pivots=piv)
 
 
 def bposd_order_decode(H, per, max_iters, osd_order, syndromes, nthreads=1, key_mode=0):
