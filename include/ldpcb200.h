@@ -77,6 +77,8 @@ typedef struct {
     int32_t kernel_rev;         /* 2: round-2 shared-memory kernel (bp_smem.cuh); 3: the same kernel with two teams per CTA taking turns
                                    in the check pass (option "dual" = 1); 1: the general persistent kernel (bp_kernel.cuh, option "lean" = 0) */
     int32_t counters_via_nccl;  /* 1: the per-device counters of a multi-device handle are summed with ncclAllReduce */
+    int64_t bpots_workspace_bytes; /* device bytes of the BP-OTS workspace of device 0 (codes beyond shared memory; allocated by
+                                      the first BP-OTS call that needs it, 0 before) */
 } ldpcb200_info_t;
 
 /* counters[] layout of the decode calls (summed over all devices of the handle) */
@@ -137,7 +139,10 @@ int ldpcb200_info(const ldpcb200_t *h, ldpcb200_info_t *out);
  *   "kernel_profile" (see ldpcb200_kernel_profile), "osd_profile"; experiments that measured no gain and stay off:
  *   "dual" (two teams per CTA), "max_ctas_per_sm";
  *   "contiguous_variables" (1, default: the shared-memory kernel gives every warp a contiguous block of variables where the
- *   code has a uniform variable degree; 0 = round-robin ownership). */
+ *   code has a uniform variable degree; 0 = round-robin ownership),
+ *   "bpots_memory" (where BP-OTS keeps the 16 E + 23 n + 4 s bytes of per-syndrome arrays: 0, default = shared memory when
+ *   they fit, otherwise a per-device workspace in global memory with one slice per resident CTA; 1 = shared memory only,
+ *   LDPCB200_EUNSUPPORTED when they do not fit; 2 = always the global workspace.  Outputs are bit-identical either way). */
 int ldpcb200_set_option(ldpcb200_t *h, const char *key, int64_t value);
 
 /* Replaces batchdecode!(decoder, syndromes, errors, success)
@@ -185,12 +190,24 @@ int ldpcb200_bposd_decode_batch(ldpcb200_t *h, int64_t B,
  * does with it.  The handle supplies H, per and max_iters (its variant is irrelevant: BP-OTS has its own Float64 LLR-domain
  * tanh/atanh updates, depolarising prior log((1 - 2 per/3)/(2 per/3)), oscillation counting, best-so-far tracking and bias -C every
  * T iterations).  errors receives best_decisions, converged the flag decode! returns, iters (nullable) the executed iterations.
- * One CTA per syndrome; both message arrays of a syndrome must fit in shared memory (LDPCB200_EUNSUPPORTED otherwise).
+ * One CTA per syndrome; its arrays live in shared memory or in the global workspace (option "bpots_memory").
  * tanh / atanh / log are CUDA's where the reference uses Julia's: outcomes agree except where a last-bit difference gets amplified. */
 int ldpcb200_bpots_decode_batch(ldpcb200_t *h, int64_t B,
                                 const void *syndromes, int32_t syn_fmt, int64_t syn_ld,
                                 void *errors, int32_t err_fmt, int64_t err_ld,
                                 uint8_t *converged, int32_t *iters, int32_t T, double C);
+
+/* The same BP-OTS decode on buffers already resident on one device of the handle, native packed rows
+ * (LDPCB200_FMT_PACKED32): d_syn_words [B][syn_words], d_err_words [B][err_words] receives best_decisions, d_converged
+ * B bytes, d_iters nullable B int32.  d_counters: nullable device pointer to LDPCB200_NUM_COUNTERS uint64; the kernel ADDS
+ * the decoded syndromes, converged ones and executed iterations to [LDPCB200_CTR_DECODED / _CONVERGED / _ITERATIONS].
+ * Asynchronous on `stream` (a cudaStream_t; NULL = the handle's own stream).  One in-flight call per handle applies in
+ * full here: codes beyond shared memory decode in a workspace shared by all BP-OTS calls on the device, so a call must have
+ * completed on its stream before another BP-OTS call of the handle is issued on a different stream. */
+int ldpcb200_bpots_device(ldpcb200_t *h, int32_t dev_slot, int64_t B,
+                          const uint32_t *d_syn_words, uint32_t *d_err_words,
+                          uint8_t *d_converged, int32_t *d_iters, unsigned long long *d_counters,
+                          int32_t T, double C, void *stream);
 
 /* The OSD-0 stage alone on device-resident buffers (native packed rows), after ldpcb200_decode_device with a
  * posterior-ratio output: d_err_words holds BP's decisions on entry and the OSD result on return;
@@ -238,6 +255,12 @@ int ldpcb200_set_per(ldpcb200_t *h, double per);
 #define LDPCB200_NUM_HARNESS_COUNTERS 8
 int ldpcb200_sample_decode_score(ldpcb200_t *h, int64_t shots, int64_t first, uint64_t seed, double per_channel,
                                  int32_t osd, int64_t *out);
+
+/* The same harness with BP-OTS (ldpcb200_bpots_decode_batch's decoder, biasing period T and constant C) in place of BP:
+ * same sampling, tiles, device shards, scoring and counter summation.  out[8] as above, with [2] the BP-OTS iterations and
+ * [7] = 0. */
+int ldpcb200_sample_bpots_score(ldpcb200_t *h, int64_t shots, int64_t first, uint64_t seed, double per_channel,
+                                int32_t T, double C, int64_t *out);
 
 /* Self-test of the kernels' branch-free division sequences against the stock IEEE routines
  * (__drcp_rn / __ddiv_rn) on n pseudo-random operands of envelope `mode` (0: t = 2/(1+q)-1,

@@ -41,3 +41,21 @@ function batchdecode!(decoder::BPOTSDecoder, syndromes::AbstractMatrix, errors::
     conv === converged || (converged .= conv)
     return errors, converged
 end
+
+"""
+    sample_decode_score(decoder::BPOTSDecoder, shots; first=0, seed=12345, per_channel=decoder.per) -> NamedTuple
+
+The sampling + scoring harness of `sample_decode_score(::BeliefPropagationDecoder, ...)` with BP-OTS as the decoder
+(ldpcb200_sample_bpots_score): errors drawn, decoded with the decoder's per, max_iters, T and C, and scored on the GPUs.
+`iterations` counts BP-OTS iterations; `osd_processed` is 0.
+"""
+function sample_decode_score(decoder::BPOTSDecoder, shots::Integer; first::Integer=0, seed::Integer=12345,
+                             per_channel::Float64=decoder.per)
+    h = _b200_ots_handle(decoder)
+    out = zeros(Int64, 8)
+    GC.@preserve out _b200_check(ccall((:ldpcb200_sample_bpots_score, LDPCB200_LIB), Cint,
+                                       (Ptr{Cvoid}, Int64, Int64, UInt64, Float64, Int32, Float64, Ptr{Int64}),
+                                       h, shots, first, UInt64(seed), per_channel, Int32(decoder.T), decoder.C, out))
+    return (shots=out[1], converged=out[2], iterations=out[3], exact_matches=out[4], syndrome_satisfied=out[5],
+            failures=out[6], residual_weight=out[7], osd_processed=out[8])
+end

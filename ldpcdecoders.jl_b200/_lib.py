@@ -25,7 +25,7 @@ SYMBOLS = [
     "ldpcb200_launch_count", "ldpcb200_selftest_division",
     "ldpcb200_bposd_decode_batch", "ldpcb200_osd0_device", "ldpcb200_kernel_profile",
     "ldpcb200_set_logicals", "ldpcb200_score_logical_device", "ldpcb200_set_per", "ldpcb200_sample_decode_score", "ldpcb200_bpots_decode_batch",
-    "ldpcb200_kernel_time",
+    "ldpcb200_kernel_time", "ldpcb200_bpots_device", "ldpcb200_sample_bpots_score",
 ]
 NUM_HARNESS_COUNTERS = 8
 HARNESS_FIELDS = ("shots", "converged", "iterations", "exact_matches", "syndrome_satisfied", "failures", "residual_weight", "osd_processed")
@@ -39,7 +39,8 @@ class Info(ctypes.Structure):
                 ("smem_bytes", ctypes.c_int32), ("slots", ctypes.c_int32),
                 ("syn_words", ctypes.c_int32), ("err_words", ctypes.c_int32),
                 ("message_bytes", ctypes.c_int64), ("kernel_mode", ctypes.c_int32), ("prefetch_distance", ctypes.c_int32),
-                ("kernel_rev", ctypes.c_int32), ("counters_via_nccl", ctypes.c_int32)]
+                ("kernel_rev", ctypes.c_int32), ("counters_via_nccl", ctypes.c_int32),
+                ("bpots_workspace_bytes", ctypes.c_int64)]
 
 
 class LibraryError(RuntimeError):
@@ -77,6 +78,8 @@ def load():
     lib.ldpcb200_sample_device.argtypes = [vp, i32, i64, i64, u64, dbl, vp, vp, vp]
     lib.ldpcb200_score_device.argtypes = [vp, i32, i64, vp, vp, vp, vp, vp]
     lib.ldpcb200_bpots_decode_batch.argtypes = [vp, i64, vp, i32, i64, vp, i32, i64, vp, vp, i32, dbl]
+    lib.ldpcb200_bpots_device.argtypes = [vp, i32, i64, vp, vp, vp, vp, vp, i32, dbl, vp]
+    lib.ldpcb200_sample_bpots_score.argtypes = [vp, i64, i64, u64, dbl, i32, dbl, ctypes.POINTER(i64)]
     lib.ldpcb200_set_logicals.argtypes = [vp, i64, vp, vp, i32]
     lib.ldpcb200_score_logical_device.argtypes = [vp, i32, i64, vp, vp, vp, vp, vp]
     lib.ldpcb200_set_per.argtypes = [vp, dbl]

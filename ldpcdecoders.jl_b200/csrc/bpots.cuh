@@ -5,8 +5,11 @@
 // :186-206, depolarising prior log((1 - 2p/3)/(2p/3)) (:231), oscillation counters, best-so-far tracking by
 // (syndrome mismatch, weight) and a bias of -C on the most oscillating / least certain variables every T iterations
 // (:294-336).  The bias step is a sequential arg-max per syndrome, so the mapping is one CTA per syndrome with threads
-// over the nodes (as bp_single.cuh), both message arrays in shared memory, block-wide lexicographic reductions for
-// the two arg-max selections.  Summation and product orders follow the reference (neighbour order, from 0.0 / 1.0), so
+// over the nodes (as bp_single.cuh), block-wide lexicographic reductions for the two arg-max selections.  The per-syndrome
+// arrays (both message arrays, node state, decisions) live in shared memory when they fit (GLOBAL = false); otherwise
+// (GLOBAL = true) each resident CTA works in its own slice of a device workspace, with the same layout and the same
+// operations in the same order, so both instantiations return bit-identical outputs.  The reduction scratch is in shared
+// memory either way.  Summation and product orders follow the reference (neighbour order, from 0.0 / 1.0), so
 // given equal tanh/atanh/log values every discrete outcome is the reference's; those three functions are CUDA's here,
 // Julia's there (see oracle/bpots_oracle.c on what that means for parity).
 #pragma once
@@ -24,7 +27,11 @@ struct BpotsParams {
     uint32_t *err_words;
     uint8_t *conv;
     int32_t *iters;
-    int off_cv, off_omega, off_llr, off_osc, off_par, off_dec, off_red;   // shared-memory byte offsets (vc at 0)
+    unsigned long long *counters;    // nullable: decoded, converged and executed iterations are ADDED to [0..2]
+    unsigned char *ws;               // GLOBAL: the workspace, one slice of slice_bytes per CTA of the grid
+    long long slice_bytes;
+    int off_cv, off_omega, off_llr, off_osc, off_par, off_dec, off_red;   // byte offsets in the per-syndrome arrays (vc at 0);
+                                                                          // off_red: of the reduction scratch in shared memory
 };
 
 constexpr int kBpotsThreads = 256;
@@ -77,16 +84,19 @@ __device__ __forceinline__ int ots_block_sum(int v, unsigned char *red_raw)
     return t;
 }
 
+template <bool GLOBAL>
 __global__ void __launch_bounds__(kBpotsThreads, 1) bpots_kernel(const BpotsParams p)
 {
     extern __shared__ __align__(16) unsigned char ots_smem[];
-    double *vc = reinterpret_cast<double *>(ots_smem);                       // [E] variable->check, then the clamped tanh of it
-    double *cv = reinterpret_cast<double *>(ots_smem + p.off_cv);            // [E] check->variable   (both in check-major slots)
-    double *omega = reinterpret_cast<double *>(ots_smem + p.off_omega);      // [n]
-    double *llr = reinterpret_cast<double *>(ots_smem + p.off_llr);          // [n]
-    int *osc = reinterpret_cast<int *>(ots_smem + p.off_osc);                // [n]
-    int *par = reinterpret_cast<int *>(ots_smem + p.off_par);                // [s] parity of the decisions on each check
-    uint8_t *dec = ots_smem + p.off_dec;                                     // [n] current, [n] previous, [n] best decisions
+    // (64-bit slice offset: grid x slice_bytes exceeds 2^31 on large codes; offsets inside a slice are below 2^31)
+    unsigned char *base = GLOBAL ? p.ws + static_cast<long long>(blockIdx.x) * p.slice_bytes : ots_smem;
+    double *vc = reinterpret_cast<double *>(base);                           // [E] variable->check, then the clamped tanh of it
+    double *cv = reinterpret_cast<double *>(base + p.off_cv);                // [E] check->variable   (both in check-major slots)
+    double *omega = reinterpret_cast<double *>(base + p.off_omega);          // [n]
+    double *llr = reinterpret_cast<double *>(base + p.off_llr);              // [n]
+    int *osc = reinterpret_cast<int *>(base + p.off_osc);                    // [n]
+    int *par = reinterpret_cast<int *>(base + p.off_par);                    // [s] parity of the decisions on each check
+    uint8_t *dec = base + p.off_dec;                                         // [n] current, [n] previous, [n] best decisions
     uint8_t *prior = dec + p.n, *best = dec + 2 * p.n;
     unsigned char *red = ots_smem + p.off_red;
     const int tid = threadIdx.x;
@@ -186,6 +196,11 @@ __global__ void __launch_bounds__(kBpotsThreads, 1) bpots_kernel(const BpotsPara
         if (tid == 0) {
             p.conv[b] = static_cast<uint8_t>(converged);
             if (p.iters) p.iters[b] = it;
+            if (p.counters) {
+                atomicAdd(&p.counters[0], 1ull);
+                atomicAdd(&p.counters[1], static_cast<unsigned long long>(converged));
+                atomicAdd(&p.counters[2], static_cast<unsigned long long>(it));
+            }
         }
         __syncthreads();
     }

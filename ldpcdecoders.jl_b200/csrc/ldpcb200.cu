@@ -172,6 +172,7 @@ struct DeviceCtx {
     long long ktime_launches = 0;
     DevBuf gk_msg, gk_state;   // grid-wide small-batch kernel (bp_grid_kernel): messages [E], resid | dec | work[2] | bar[2]
     int gk_blocks_per_sm = -1; // its co-resident CTAs per SM (-1: not asked yet, 0: unavailable)
+    DevBuf bpots_ws;        // BP-OTS arrays of codes beyond shared memory: one slice per resident CTA (see bpots_on_device)
     DevBuf tiny;            // small-batch host calls: one device block ...
     PinnedBuf tiny_host;    // ... mirrored by one pinned block (one copy each way, one synchronisation)
 };
@@ -219,6 +220,7 @@ struct ldpcb200 {
     int opt_time_kernels = 0;    // bracket every launch of the decoding kernel with CUDA events (ldpcb200_kernel_time)
     int opt_max_ctas = 0;        // cap on resident CTAs per SM (0: whatever fits; experiments)
     int opt_lean = 1;            // family SMEM: use the round-2 kernel (bp_smem.cuh) when the code fits its envelope
+    int opt_bpots_memory = 0;    // BP-OTS arrays: 0 shared memory where they fit, else the global workspace; 1 shared only; 2 global
     // resolved configuration
     bool configured = false;
     int family = 0, mode = 0, warps = 0, ctas_per_sm = 0, smem_bytes = 0, slots = 0, shape = 0;
@@ -551,7 +553,7 @@ void destroy_device(DeviceCtx &d)
     cudaFree(d.d_p_rowptr); cudaFree(d.d_p_colptr); cudaFree(d.d_corig); cudaFree(d.d_vorig);
     if (d.set[1].stream) cudaStreamSynchronize(d.set[1].stream);
     for (DevBuf *b : {&d.gk_msg, &d.gk_state, &d.msg, &d.state, &d.efield, &d.counters, &d.scratch, &d.osd_stats, &d.tiny, &d.kprof, &d.ctr_sum, &d.f_vars, &d.f_edeg, &d.f_epos, &d.f_ctab, &d.f_list, &d.f_count, &d.lmask, &d.hs_truth, &d.hs_syn, &d.hs_err,
-                       &d.hs_conv, &d.hs_iters, &d.hs_ratio, &d.hs_ctr, &d.hs_sum}) b->release();
+                       &d.hs_conv, &d.hs_iters, &d.hs_ratio, &d.hs_ctr, &d.hs_sum, &d.bpots_ws}) b->release();
     d.tiny_host.release();
     for (auto &S : d.set)
         for (DevBuf *b : {&S.raw_in, &S.raw_out, &S.syn_words, &S.err_words, &S.conv, &S.iters, &S.ratio, &S.osd_list, &S.osd_ctl, &S.f_list, &S.f_count})
@@ -1162,10 +1164,14 @@ int osdk_on_device(ldpcb200 *h, DeviceCtx &d, DeviceCtx::StageSet &S, int64_t B,
 }
 
 // ---- BP-OTS (bpots.cuh): one CTA per syndrome.  Stream-ordered.
+// The per-syndrome arrays (16 E + 23 n + 4 s bytes) live in shared memory when they fit; otherwise every CTA of the grid
+// gets its own slice of the device's workspace d.bpots_ws.  That workspace is shared by all BP-OTS launches on the device:
+// launches that use it must not overlap (host-batch chunks are ordered by decode_done; device-resident calls follow the
+// one-in-flight-call-per-handle rule).
 struct BpotsArgs { int T; double C; };
 
 int bpots_on_device(ldpcb200 *h, DeviceCtx &d, int64_t B, const uint32_t *syn_words, uint32_t *err_words, uint8_t *conv, int32_t *iters,
-                    const BpotsArgs &a, cudaStream_t st)
+                    const BpotsArgs &a, unsigned long long *counters, cudaStream_t st)
 {
     if (B <= 0) return 0;
     CU(cudaSetDevice(d.device));
@@ -1186,17 +1192,40 @@ int bpots_on_device(ldpcb200 *h, DeviceCtx &d, int64_t B, const uint32_t *syn_wo
     p.off_par = static_cast<int>(off);    off += static_cast<long long>(std::max<int64_t>(h->s, 1)) * 4;
     p.off_dec = static_cast<int>(off);    off += 3 * std::max<int64_t>(h->n, 1);
     off = (off + 15) / 16 * 16;
-    p.off_red = static_cast<int>(off);    off += 512;
-    if (off > d.smem_optin)
-        return fail(LDPCB200_EUNSUPPORTED, "BP-OTS: the two message arrays of one syndrome (%lld bytes with state) do not fit in shared memory",
-                    off);
-    const int smem = static_cast<int>(off);
+    const long long arrays = off;                     // bytes of the per-syndrome arrays
+    if (arrays > 0x7fffffffLL)
+        return fail(LDPCB200_EUNSUPPORTED, "BP-OTS: the arrays of one syndrome (%lld bytes) exceed 2^31 bytes", arrays);
+    const bool fits = arrays + 512 <= d.smem_optin;
+    if (h->opt_bpots_memory == 1 && !fits)
+        return fail(LDPCB200_EUNSUPPORTED, "BP-OTS: the two message arrays of one syndrome (%lld bytes with state) do not fit in shared memory "
+                    "(option bpots_memory = 1)", arrays + 512);
     p.rowptr = d.d_rowptr; p.colptr = d.d_colptr; p.ve_slot = d.d_ve_slot; p.ve_chk = d.d_ve_chk;
-    p.syn_words = syn_words; p.err_words = err_words; p.conv = conv; p.iters = iters;
-    const int per_sm = std::max(1, std::min(8, d.smem_per_sm / (smem + 1024)));
-    const int grid = static_cast<int>(std::min<int64_t>(B, static_cast<int64_t>(d.sm_count) * per_sm));
-    CU(cudaFuncSetAttribute(bp::bpots_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    bp::bpots_kernel<<<grid, bp::kBpotsThreads, smem, st>>>(p);
+    p.syn_words = syn_words; p.err_words = err_words; p.conv = conv; p.iters = iters; p.counters = counters;
+    if (fits && h->opt_bpots_memory != 2) {
+        p.off_red = static_cast<int>(arrays);
+        const int smem = static_cast<int>(arrays + 512);
+        const int per_sm = std::max(1, std::min(8, d.smem_per_sm / (smem + 1024)));
+        const int grid = static_cast<int>(std::min<int64_t>(B, static_cast<int64_t>(d.sm_count) * per_sm));
+        CU(cudaFuncSetAttribute(bp::bpots_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        bp::bpots_kernel<false><<<grid, bp::kBpotsThreads, smem, st>>>(p);
+    } else {
+        // grid: resident CTAs, at most one per syndrome, and at most a quarter of the free device memory in slices
+        const long long slice = (arrays + 255) / 256 * 256;
+        int occ = 0;
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, bp::bpots_kernel<true>, bp::kBpotsThreads, 512));
+        size_t free_b = 0, total_b = 0;
+        CU(cudaMemGetInfo(&free_b, &total_b));
+        const long long cap = static_cast<long long>((free_b + d.bpots_ws.cap) / 4);
+        if (slice > cap)
+            return fail(LDPCB200_ENOMEM, "BP-OTS: the workspace of one syndrome (%lld bytes) exceeds a quarter of the free device memory", slice);
+        const int grid = static_cast<int>(std::min<int64_t>({B, static_cast<int64_t>(d.sm_count) * std::max(occ, 1), cap / slice}));
+        int rc = d.bpots_ws.reserve(static_cast<size_t>(grid) * static_cast<size_t>(slice));
+        if (rc) return rc;
+        p.ws = d.bpots_ws.as<unsigned char>();
+        p.slice_bytes = slice;
+        p.off_red = 0;
+        bp::bpots_kernel<true><<<grid, bp::kBpotsThreads, 512, st>>>(p);
+    }
     h->launches++;
     CU(cudaGetLastError());
     return 0;
@@ -1474,7 +1503,8 @@ int decode_host_range(ldpcb200 *h, DeviceCtx &d, int64_t b0, int64_t Bd, int64_t
         // (OSD-0 only reads the ratios of unconverged syndromes: those of iteration max_iters; a higher order post-processes
         //  every syndrome, so the ratios of each syndrome's own last iteration are needed)
         if (ots)
-            rc = bpots_on_device(h, d, Bc, syn_words, S.err_words.as<uint32_t>(), S.conv.as<uint8_t>(), S.iters.as<int32_t>(), *ots, st);
+            rc = bpots_on_device(h, d, Bc, syn_words, S.err_words.as<uint32_t>(), S.conv.as<uint8_t>(), S.iters.as<int32_t>(), *ots,
+                                 nullptr, st);
         else
         rc = decode_on_device(h, d, Bc, syn_words, S.err_words.as<uint32_t>(), S.conv.as<uint8_t>(), S.iters.as<int32_t>(),
                               (ratio || (osd && h->max_iters > 0)) ? S.ratio.as<double>() : nullptr,
@@ -1617,8 +1647,9 @@ int nccl_sum_counters(ldpcb200 *h, int64_t *out)
 }
 
 // One device's share of the sampling + scoring harness: tiles of device-resident shots.
+// ots: BP-OTS instead of BP (osd is then false).
 int harness_on_device(ldpcb200 *h, DeviceCtx &d, int64_t first, int64_t shots, uint64_t seed, double per_channel, bool osd,
-                      int64_t *out8)
+                      const BpotsArgs *ots, int64_t *out8)
 {
     CU(cudaSetDevice(d.device));
     cudaStream_t st = d.set[0].stream;
@@ -1655,8 +1686,12 @@ int harness_on_device(ldpcb200 *h, DeviceCtx &d, int64_t first, int64_t shots, u
                                                                              d.hs_syn.as<uint32_t>());
             h->launches += 2;
             const bool want_ratio = osd && h->max_iters > 0;
-            rc = decode_on_device(h, d, bt, d.hs_syn.as<uint32_t>(), d.hs_err.as<uint32_t>(), d.hs_conv.as<uint8_t>(), d.hs_iters.as<int32_t>(),
-                                  want_ratio ? d.hs_ratio.as<double>() : nullptr, ctr + LDPCB200_NUM_HARNESS_COUNTERS, st, h->opt_osd_order == 0);
+            if (ots)
+                rc = bpots_on_device(h, d, bt, d.hs_syn.as<uint32_t>(), d.hs_err.as<uint32_t>(), d.hs_conv.as<uint8_t>(), d.hs_iters.as<int32_t>(),
+                                     *ots, ctr + LDPCB200_NUM_HARNESS_COUNTERS, st);
+            else
+                rc = decode_on_device(h, d, bt, d.hs_syn.as<uint32_t>(), d.hs_err.as<uint32_t>(), d.hs_conv.as<uint8_t>(), d.hs_iters.as<int32_t>(),
+                                      want_ratio ? d.hs_ratio.as<double>() : nullptr, ctr + LDPCB200_NUM_HARNESS_COUNTERS, st, h->opt_osd_order == 0);
             if (rc) return rc;
             if (osd) {
                 if (h->max_iters <= 0) {
@@ -1804,6 +1839,11 @@ int ldpcb200_set_option(ldpcb200_t *h, const char *key, int64_t value)
     else if (k == "prefetch") h->opt_pd = static_cast<int>(value);
     else if (k == "ring_mult") h->opt_ring_mult = static_cast<int>(std::min<int64_t>(std::max<int64_t>(value, 0), 4));
     else if (k == "lean") h->opt_lean = value ? 1 : 0;
+    else if (k == "bpots_memory") {
+        if (value < 0 || value > 2) return fail(LDPCB200_EINVAL, "bpots_memory must be 0 (auto), 1 (shared) or 2 (global)");
+        h->opt_bpots_memory = static_cast<int>(value);
+        return 0;
+    }
     else if (k == "first_iteration_filter") { h->opt_filter = value ? 1 : 0; return 0; }
     else if (k == "dual") h->opt_dual = value ? 1 : 0;
     else if (k == "contiguous_variables") h->opt_cv = value ? 1 : 0;
@@ -1838,6 +1878,7 @@ int ldpcb200_info(const ldpcb200_t *hc, ldpcb200_info_t *out)
     out->kernel_rev = h->lean ? (h->dual ? 3 : 2) : 1;
     nccl_prepare(h);
     out->counters_via_nccl = h->nccl_state == 1 ? 1 : 0;
+    out->bpots_workspace_bytes = static_cast<int64_t>(h->dev[0].bpots_ws.cap);
     return 0;
 }
 
@@ -1944,6 +1985,18 @@ int ldpcb200_bpots_decode_batch(ldpcb200_t *h, int64_t B, const void *syndromes,
 {
     const BpotsArgs a{T, C};
     return decode_batch_impl(h, B, syndromes, syn_fmt, syn_ld, errors, err_fmt, err_ld, converged, iters, nullptr, nullptr, false, nullptr, &a);
+}
+
+int ldpcb200_bpots_device(ldpcb200_t *h, int32_t dev_slot, int64_t B, const uint32_t *d_syn_words, uint32_t *d_err_words,
+                          uint8_t *d_converged, int32_t *d_iters, unsigned long long *d_counters, int32_t T, double C, void *stream)
+{
+    if (!h) return fail(LDPCB200_EINVAL, "null handle");
+    if (dev_slot < 0 || dev_slot >= static_cast<int>(h->dev.size())) return fail(LDPCB200_EINVAL, "bad dev_slot");
+    if (B < 0 || (B > 0 && (!d_syn_words || !d_err_words || !d_converged))) return fail(LDPCB200_EINVAL, "null device buffer");
+    DeviceCtx &d = h->dev[dev_slot];
+    const BpotsArgs a{T, C};
+    return bpots_on_device(h, d, B, d_syn_words, d_err_words, d_converged, d_iters, a, d_counters,
+                           stream ? static_cast<cudaStream_t>(stream) : d.stream);
 }
 
 int ldpcb200_osd0_device(ldpcb200_t *h, int32_t dev_slot, int64_t B, const uint32_t *d_syn_words, uint32_t *d_err_words,
@@ -2067,8 +2120,8 @@ int ldpcb200_set_per(ldpcb200_t *h, double per)
     return 0;
 }
 
-int ldpcb200_sample_decode_score(ldpcb200_t *h, int64_t shots, int64_t first, uint64_t seed, double per_channel, int32_t osd,
-                                 int64_t *out)
+static int sample_score_impl(ldpcb200_t *h, int64_t shots, int64_t first, uint64_t seed, double per_channel, int32_t osd,
+                             const BpotsArgs *ots, int64_t *out)
 {
     if (!h || !out) return fail(LDPCB200_EINVAL, "null argument");
     memset(out, 0, sizeof(int64_t) * LDPCB200_NUM_HARNESS_COUNTERS);
@@ -2086,7 +2139,7 @@ int ldpcb200_sample_decode_score(ldpcb200_t *h, int64_t shots, int64_t first, ui
     std::vector<std::string> errs(nd);
     std::vector<int64_t> ctr(static_cast<size_t>(nd) * LDPCB200_NUM_HARNESS_COUNTERS, 0);
     auto work = [&](int k) {
-        rcs[k] = harness_on_device(h, h->dev[k], first + lo[k], lo[k + 1] - lo[k], seed, per_channel, osd != 0,
+        rcs[k] = harness_on_device(h, h->dev[k], first + lo[k], lo[k + 1] - lo[k], seed, per_channel, osd != 0, ots,
                                    &ctr[static_cast<size_t>(k) * LDPCB200_NUM_HARNESS_COUNTERS]);
         if (rcs[k]) errs[k] = g_err;
     };
@@ -2112,6 +2165,19 @@ int ldpcb200_sample_decode_score(ldpcb200_t *h, int64_t shots, int64_t first, ui
         for (int k = 0; k < nd; ++k)
             for (int c = 0; c < LDPCB200_NUM_HARNESS_COUNTERS; ++c) out[c] += ctr[static_cast<size_t>(k) * LDPCB200_NUM_HARNESS_COUNTERS + c];
     return 0;
+}
+
+int ldpcb200_sample_decode_score(ldpcb200_t *h, int64_t shots, int64_t first, uint64_t seed, double per_channel, int32_t osd,
+                                 int64_t *out)
+{
+    return sample_score_impl(h, shots, first, seed, per_channel, osd, nullptr, out);
+}
+
+int ldpcb200_sample_bpots_score(ldpcb200_t *h, int64_t shots, int64_t first, uint64_t seed, double per_channel, int32_t T, double C,
+                                int64_t *out)
+{
+    const BpotsArgs a{T, C};
+    return sample_score_impl(h, shots, first, seed, per_channel, 0, &a, out);
 }
 
 int ldpcb200_selftest_division(int32_t device, int32_t mode, uint64_t n, uint64_t seed, uint64_t *mismatches)

@@ -229,6 +229,31 @@ class BPOTSDecoder:
             self._bp._h, int(B), syn.ctypes.data, syn_fmt, int(syn_ld), err.ctypes.data, err_fmt, int(err_ld), conv.ctypes.data,
             iters.ctypes.data if iters is not None else None, self.T, self.C))
 
+    def decode_device(self, B, d_syn_words, d_err_words, d_conv, d_iters=None, d_counters=None, stream=None, dev_slot=0):
+        """BP-OTS on device-resident packed rows (ldpcb200_bpots_device), asynchronous on `stream`; d_counters (nullable,
+        four uint64) receives ADDED decoded / converged / iteration counts."""
+        _lib.check(self._bp._lib.ldpcb200_bpots_device(self._bp._h, dev_slot, int(B), d_syn_words, d_err_words, d_conv, d_iters,
+                                                       d_counters, self.T, self.C, stream))
+
+    def sample_decode_score(self, shots, first, seed, per_channel):
+        """The sampling + scoring harness with BP-OTS as the decoder (ldpcb200_sample_bpots_score); returns a dict of the
+        eight counters (iterations = BP-OTS iterations, osd_processed = 0)."""
+        out = (ctypes.c_int64 * _lib.NUM_HARNESS_COUNTERS)()
+        _lib.check(self._bp._lib.ldpcb200_sample_bpots_score(self._bp._h, int(shots), int(first), ctypes.c_uint64(seed),
+                                                             float(per_channel), self.T, self.C, out))
+        return dict(zip(_lib.HARNESS_FIELDS, [int(x) for x in out]))
+
+    def set_per(self, per):
+        """New prior for the same device-resident Tanner graph (the depolarising prior follows it)."""
+        self._bp.set_per(per)
+        self.per = self._bp.per
+
+    def set_logicals(self, L):
+        self._bp.set_logicals(L)
+
+    def set_option(self, key, value):
+        self._bp.set_option(key, value)
+
     def info(self):
         return self._bp.info()
 
@@ -345,15 +370,22 @@ def ler_curve(decoder, pers, shots, seed=12345, osd=False, match_prior=True):
     """Logical-error-rate sweep on the GPU (the loop of test/test_bp_decoder.jl:19-30 per error rate, with the batch
     sampled, decoded and scored on the device): for each physical error rate the prior is set to it (match_prior), `shots`
     errors are drawn from the Philox stream, decoded (BP, or BP+OSD-0 with osd=True) and compared with the truth.
+    A BPOTSDecoder is swept with BP-OTS as the decoder (osd does not apply).
     Returns one dict per rate: the eight counters plus ler (= failures / shots), converged_frac and mean_iters."""
     bp = decoder.bp_decoder if isinstance(decoder, BeliefPropagationOSDDecoder) else decoder
+    ots = isinstance(decoder, BPOTSDecoder)
+    if ots and osd:
+        raise ValueError("osd does not apply to the BP-OTS decoder")
     osd = osd or isinstance(decoder, BeliefPropagationOSDDecoder)
     prior = bp.per
     rows = []
     for k, per in enumerate(pers):
         if match_prior:
             bp.set_per(per)
-        c = bp.sample_decode_score(shots, k * int(shots), seed, per, osd=osd)
+        if ots:
+            c = bp.sample_decode_score(shots, k * int(shots), seed, per)
+        else:
+            c = bp.sample_decode_score(shots, k * int(shots), seed, per, osd=osd)
         c.update(per=float(per), ler=c["failures"] / max(c["shots"], 1), converged_frac=c["converged"] / max(c["shots"], 1),
                  mean_iters=c["iterations"] / max(c["shots"], 1))
         rows.append(c)
