@@ -246,6 +246,24 @@ namespace {
 
 inline int align_up(int x, int a) { return (x + a - 1) / a * a; }
 
+inline int grid_for(long long work, int sm) { return static_cast<int>(std::max<long long>(1, std::min<long long>((work + 255) / 256, static_cast<long long>(sm) * 16))); }
+
+// channel_probs[j] / (1 - channel_probs[j]) (belief_propagation.jl:129,153), IEEE double on the host
+void set_prior(ldpcb200 *h, double per)
+{
+    volatile double one_minus = 1.0 - per;
+    volatile double q = per / one_minus;
+    h->per = per;
+    for (DeviceCtx &d : h->dev) d.f_ready = false;        // the first-iteration tables depend on the prior
+    h->p0 = q;
+    h->regular_p0 = std::isnormal(h->p0) && h->p0 > 0.0;
+    if (h->variant != LDPCB200_VARIANT_EXACT) {         // the kernels' prior slot carries L0 = log((1-p)/p)
+        volatile double r = one_minus / per;
+        h->p0 = std::log(r);
+        if (h->variant == LDPCB200_VARIANT_FAST32) h->p0 = static_cast<double>(static_cast<float>(h->p0));
+    }
+}
+
 // shared-memory carve-up for a kernel mode / thread count; returns total bytes
 //   mode 0: messages | syn | resid | stage | nnz | [efield] | tables | mbar
 //   mode 1:            syn | resid | stage | nnz | [efield] | tables | mbar
@@ -559,6 +577,8 @@ void destroy_device(DeviceCtx &d)
         for (DevBuf *b : {&S.raw_in, &S.raw_out, &S.syn_words, &S.err_words, &S.conv, &S.iters, &S.ratio, &S.osd_list, &S.osd_ctl, &S.f_list, &S.f_count})
             b->release();
     for (auto &S : d.set) { S.pin_in.release(); S.pin_out.release(); }
+    for (auto &pr : d.ktime_events) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); }   // not yet read by ldpcb200_kernel_time
+    d.ktime_events.clear();
     if (d.decode_done) cudaEventDestroy(d.decode_done);
     if (d.set[1].stream) cudaStreamDestroy(d.set[1].stream);
     if (d.stream) cudaStreamDestroy(d.stream);
@@ -577,64 +597,39 @@ int kernel_shape(bool two_ctas, int threads, int mode = 0, bool big = false)
     return kShape384x2;
 }
 
-// The (MODE, BIG, VARIANT) instantiations live in their own translation units (bp_inst_*.cu).
-int kernel_attrs_dispatch(int variant, int mode, bool big, int shape, int smem_bytes, int threads, int *bps)
-{
-    cudaError_t e;
-    if (variant == LDPCB200_VARIANT_MINSUM) {
-        switch (mode) {
-            case 0: e = bp::kernel_attrs_0_0_1(shape, smem_bytes, threads, bps); break;
-            case 1: e = bp::kernel_attrs_1_0_1(shape, smem_bytes, threads, bps); break;
-            default: e = bp::kernel_attrs_2_0_1(shape, smem_bytes, threads, bps); break;
-        }
-    } else if (variant == LDPCB200_VARIANT_FAST32) {
-        switch (mode) {
-            case 0: e = bp::kernel_attrs_0_0_2(shape, smem_bytes, threads, bps); break;
-            case 1: e = bp::kernel_attrs_1_0_2(shape, smem_bytes, threads, bps); break;
-            default: e = bp::kernel_attrs_2_0_2(shape, smem_bytes, threads, bps); break;
-        }
-    } else {
-        switch (mode * 2 + (big ? 1 : 0)) {
-            case 0: e = bp::kernel_attrs_0_0_0(shape, smem_bytes, threads, bps); break;
-            case 1: e = bp::kernel_attrs_0_1_0(shape, smem_bytes, threads, bps); break;
-            case 2: e = bp::kernel_attrs_1_0_0(shape, smem_bytes, threads, bps); break;
-            case 3: e = bp::kernel_attrs_1_1_0(shape, smem_bytes, threads, bps); break;
-            case 4: e = bp::kernel_attrs_2_0_0(shape, smem_bytes, threads, bps); break;
-            default: e = bp::kernel_attrs_2_1_0(shape, smem_bytes, threads, bps); break;
-        }
-    }
-    if (e != cudaSuccess) return fail(LDPCB200_ECUDA, "kernel attributes (mode %d): %s", mode, cudaGetErrorString(e));
-    return 0;
-}
+// The compiled kernels of one variant.  The instantiations live in their own translation units (bp_inst_*.cu); the
+// persistent kernel's are indexed [mode][big], nullptr where none exists (the min-sum and fast variants have no
+// local-memory degree path: ldpcb200_create refuses those codes).
+struct VariantKernels {
+    decltype(&bp::kernel_attrs_0_0_0) attrs[3][2];
+    decltype(&bp::kernel_launch_0_0_0) launch[3][2];
+    decltype(&bp::smem_kernel_attrs_0) smem_attrs;
+    decltype(&bp::smem_kernel_launch_0) smem_launch;
+    decltype(&bp::smem_dual_attrs_0) dual_attrs;
+    decltype(&bp::smem_dual_launch_0) dual_launch;
+    decltype(&bp::filter_setup_0) filter_setup;
+    decltype(&bp::grid_kernel_occupancy_0) grid_occupancy;
+    decltype(&bp::grid_launch_0) grid_launch;
+    decltype(&bp::single_launch_0) single_launch;
+};
 
-void kernel_launch_dispatch(int variant, int mode, bool big, int shape, int grid, int threads, int smem_bytes, cudaStream_t st,
-                            const bp::KernelParams &p)
-{
-    if (variant == LDPCB200_VARIANT_MINSUM) {
-        switch (mode) {
-            case 0: bp::kernel_launch_0_0_1(shape, grid, threads, smem_bytes, st, p); break;
-            case 1: bp::kernel_launch_1_0_1(shape, grid, threads, smem_bytes, st, p); break;
-            default: bp::kernel_launch_2_0_1(shape, grid, threads, smem_bytes, st, p); break;
-        }
-        return;
-    }
-    if (variant == LDPCB200_VARIANT_FAST32) {
-        switch (mode) {
-            case 0: bp::kernel_launch_0_0_2(shape, grid, threads, smem_bytes, st, p); break;
-            case 1: bp::kernel_launch_1_0_2(shape, grid, threads, smem_bytes, st, p); break;
-            default: bp::kernel_launch_2_0_2(shape, grid, threads, smem_bytes, st, p); break;
-        }
-        return;
-    }
-    switch (mode * 2 + (big ? 1 : 0)) {
-        case 0: bp::kernel_launch_0_0_0(shape, grid, threads, smem_bytes, st, p); break;
-        case 1: bp::kernel_launch_0_1_0(shape, grid, threads, smem_bytes, st, p); break;
-        case 2: bp::kernel_launch_1_0_0(shape, grid, threads, smem_bytes, st, p); break;
-        case 3: bp::kernel_launch_1_1_0(shape, grid, threads, smem_bytes, st, p); break;
-        case 4: bp::kernel_launch_2_0_0(shape, grid, threads, smem_bytes, st, p); break;
-        default: bp::kernel_launch_2_1_0(shape, grid, threads, smem_bytes, st, p); break;
-    }
-}
+const VariantKernels kVariantKernels[3] = {
+    {{{bp::kernel_attrs_0_0_0, bp::kernel_attrs_0_1_0}, {bp::kernel_attrs_1_0_0, bp::kernel_attrs_1_1_0}, {bp::kernel_attrs_2_0_0, bp::kernel_attrs_2_1_0}},
+     {{bp::kernel_launch_0_0_0, bp::kernel_launch_0_1_0}, {bp::kernel_launch_1_0_0, bp::kernel_launch_1_1_0}, {bp::kernel_launch_2_0_0, bp::kernel_launch_2_1_0}},
+     bp::smem_kernel_attrs_0, bp::smem_kernel_launch_0, bp::smem_dual_attrs_0, bp::smem_dual_launch_0, bp::filter_setup_0,
+     bp::grid_kernel_occupancy_0, bp::grid_launch_0, bp::single_launch_0},
+    {{{bp::kernel_attrs_0_0_1, nullptr}, {bp::kernel_attrs_1_0_1, nullptr}, {bp::kernel_attrs_2_0_1, nullptr}},
+     {{bp::kernel_launch_0_0_1, nullptr}, {bp::kernel_launch_1_0_1, nullptr}, {bp::kernel_launch_2_0_1, nullptr}},
+     bp::smem_kernel_attrs_1, bp::smem_kernel_launch_1, bp::smem_dual_attrs_1, bp::smem_dual_launch_1, bp::filter_setup_1,
+     bp::grid_kernel_occupancy_1, bp::grid_launch_1, bp::single_launch_1},
+    {{{bp::kernel_attrs_0_0_2, nullptr}, {bp::kernel_attrs_1_0_2, nullptr}, {bp::kernel_attrs_2_0_2, nullptr}},
+     {{bp::kernel_launch_0_0_2, nullptr}, {bp::kernel_launch_1_0_2, nullptr}, {bp::kernel_launch_2_0_2, nullptr}},
+     bp::smem_kernel_attrs_2, bp::smem_kernel_launch_2, bp::smem_dual_attrs_2, bp::smem_dual_launch_2, bp::filter_setup_2,
+     bp::grid_kernel_occupancy_2, bp::grid_launch_2, bp::single_launch_2},
+};
+
+// (indexed by LDPCB200_VARIANT_*, which ldpcb200_create checks)
+const VariantKernels &kernels_of(int variant) { return kVariantKernels[variant]; }
 
 // Warps per CTA: warp w owns checks w, w+W, ... and variables w, w+W, ...; pick the W whose two
 // round-robin splits waste the fewest warp-slots (ties -> more warps, better latency hiding).
@@ -774,20 +769,16 @@ int configure(ldpcb200 *h)
         h->tables_dirty = false;
         CU(cudaSetDevice(d0.device));
     }
-    int bps = 0, rc;
+    const VariantKernels &K = kernels_of(h->variant);
+    int bps = 0;
     for (DeviceCtx &d : h->dev) {
         CU(cudaSetDevice(d.device));
         if (lean) {
-            cudaError_t e;
-            const int v = h->variant;
-            if (dual) e = v == 1 ? bp::smem_dual_attrs_1(eb64, need, 2 * warps * 32, &bps)
-                        : v == 2 ? bp::smem_dual_attrs_2(eb64, need, 2 * warps * 32, &bps) : bp::smem_dual_attrs_0(eb64, need, 2 * warps * 32, &bps);
-            else e = v == 1 ? bp::smem_kernel_attrs_1(shape, eb64, need, warps * 32, &bps)
-                   : v == 2 ? bp::smem_kernel_attrs_2(shape, eb64, need, warps * 32, &bps) : bp::smem_kernel_attrs_0(shape, eb64, need, warps * 32, &bps);
+            cudaError_t e = dual ? K.dual_attrs(eb64, need, 2 * warps * 32, &bps) : K.smem_attrs(shape, eb64, need, warps * 32, &bps);
             if (e != cudaSuccess) return fail(LDPCB200_ECUDA, "kernel attributes (shared-memory kernel): %s", cudaGetErrorString(e));
         } else {
-            rc = kernel_attrs_dispatch(h->variant, mode, h->big, shape, need, warps * 32, &bps);
-            if (rc) return rc;
+            cudaError_t e = K.attrs[mode][h->big](shape, need, warps * 32, &bps);
+            if (e != cudaSuccess) return fail(LDPCB200_ECUDA, "kernel attributes (mode %d): %s", mode, cudaGetErrorString(e));
         }
     }
     if (bps < 1) return fail(LDPCB200_EUNSUPPORTED, "BP kernel (mode %d, %d threads, %d B smem) does not fit on an SM", mode, warps * 32, need);
@@ -837,8 +828,7 @@ int filter_prepare(ldpcb200 *h, DeviceCtx &d, cudaStream_t st)
     q.n = static_cast<int>(n); q.p0 = h->p0; q.check_aux = h->ms_scale; q.regular_p0 = h->regular_p0;
     q.colptr = d.d_colptr; q.e_deg = d.f_edeg.as<uint8_t>(); q.e_pos = d.f_epos.as<uint8_t>();
     q.ctab = d.f_ctab.as<double>(); q.vars = d.f_vars.as<bp::FilterVar>();
-    cudaError_t e = h->variant == LDPCB200_VARIANT_MINSUM ? bp::filter_setup_1(q, st)
-                  : h->variant == LDPCB200_VARIANT_FAST32 ? bp::filter_setup_2(q, st) : bp::filter_setup_0(q, st);
+    cudaError_t e = kernels_of(h->variant).filter_setup(q, st);
     if (e != cudaSuccess) return fail(LDPCB200_ECUDA, "first-iteration tables: %s", cudaGetErrorString(e));
     CU(cudaStreamSynchronize(st));              // (other streams of the device read the tables from now on)
     h->launches += 2;
@@ -887,19 +877,26 @@ int decode_on_device(ldpcb200 *h, DeviceCtx &d, int64_t B, const uint32_t *syn_w
         }
         return 0;
     }
+    const VariantKernels &K = kernels_of(h->variant);
     // ---- small batches: one CTA per syndrome, threads over the nodes (bp_single.cuh)
     {
         const int64_t limit = h->opt_small_batch < 0 ? d.sm_count : h->opt_small_batch;
         const int off_syn = static_cast<int>((std::max<int64_t>(h->E, 1) * 8 + 15) / 16 * 16);
         const int smem = off_syn + 2 * h->SW * 4 + h->NW * 4;
+        auto common = [&](auto &q) {        // the fields bp::SingleParams and bp::GridParams share
+            q.s = static_cast<int>(h->s); q.n = static_cast<int>(h->n); q.E = static_cast<int>(h->E);
+            q.SW = h->SW; q.NW = h->NW; q.max_iters = h->max_iters; q.early_stop = h->opt_early_stop;
+            q.regular_p0 = h->regular_p0; q.ratio_last_only = ratio_last_only ? 1 : 0; q.p0 = h->p0; q.check_aux = h->ms_scale; q.B = B;
+            q.rowptr = d.d_rowptr; q.colptr = d.d_colptr; q.ve_slot = d.d_ve_slot; q.ve_chk = d.d_ve_chk;
+            q.syn_words = syn_words; q.err_words = err_words; q.conv = conv; q.iters = iters; q.ratio = ratio; q.counters = counters;
+        };
         // ... or, when the messages of one syndrome do not fit in an SM's shared memory, the whole grid per syndrome
         // (cooperative launch, messages in L2): otherwise a lone decode! on a large code walks every edge on ONE lane
         if (B <= limit && !h->big && (smem > d.smem_optin || h->opt_grid_kernel == 2) && h->E > 0) {   // (2: always, a test hook)
             if (d.gk_blocks_per_sm < 0) {
                 int coop = 0, bps = 0;
                 cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, d.device);
-                cudaError_t e = h->variant == LDPCB200_VARIANT_MINSUM ? bp::grid_kernel_occupancy_1(&bps)
-                              : h->variant == LDPCB200_VARIANT_FAST32 ? bp::grid_kernel_occupancy_2(&bps) : bp::grid_kernel_occupancy_0(&bps);
+                cudaError_t e = K.grid_occupancy(&bps);
                 if (e != cudaSuccess) { cudaGetLastError(); bps = 0; }
                 d.gk_blocks_per_sm = coop ? bps : 0;
             }
@@ -914,32 +911,20 @@ int decode_on_device(ldpcb200 *h, DeviceCtx &d, int64_t B, const uint32_t *syn_w
                 if ((rc = d.gk_msg.reserve(static_cast<size_t>(h->E) * 8)) || (rc = d.gk_state.reserve(st_bytes))) return rc;
                 if (fresh_state) CU(cudaMemsetAsync(d.gk_state.p, 0, st_bytes, st));      // counters start at zero; the kernel leaves them so
                 bp::GridParams q{};
-                q.s = static_cast<int>(h->s); q.n = static_cast<int>(h->n); q.E = static_cast<int>(h->E);
-                q.SW = h->SW; q.NW = h->NW; q.max_iters = h->max_iters; q.early_stop = h->opt_early_stop;
-                q.regular_p0 = h->regular_p0; q.ratio_last_only = ratio_last_only ? 1 : 0; q.p0 = h->p0; q.check_aux = h->ms_scale; q.B = B;
-                q.rowptr = d.d_rowptr; q.colptr = d.d_colptr; q.ve_slot = d.d_ve_slot; q.ve_chk = d.d_ve_chk;
-                q.syn_words = syn_words; q.err_words = err_words; q.conv = conv; q.iters = iters; q.ratio = ratio; q.counters = counters;
+                common(q);
                 q.msg = d.gk_msg.as<double>();
                 q.resid = d.gk_state.as<uint32_t>(); q.dec = q.resid + h->SW;
                 q.work = reinterpret_cast<int *>(q.dec + h->NW); q.bar = reinterpret_cast<unsigned int *>(q.work + 2);
-                CU(h->variant == LDPCB200_VARIANT_MINSUM ? bp::grid_launch_1(grid, st, q)
-                   : h->variant == LDPCB200_VARIANT_FAST32 ? bp::grid_launch_2(grid, st, q) : bp::grid_launch_0(grid, st, q));
+                CU(K.grid_launch(grid, st, q));
                 h->launches++;
                 return 0;
             }
         }
         if (B <= limit && !h->big && smem <= d.smem_optin && h->E * 8 < (1 << 30)) {
             bp::SingleParams q{};
-            q.s = static_cast<int>(h->s); q.n = static_cast<int>(h->n); q.E = static_cast<int>(h->E);
-            q.SW = h->SW; q.NW = h->NW; q.max_iters = h->max_iters; q.early_stop = h->opt_early_stop;
-            q.regular_p0 = h->regular_p0; q.ratio_last_only = ratio_last_only ? 1 : 0; q.p0 = h->p0; q.check_aux = h->ms_scale; q.B = B;
-            q.rowptr = d.d_rowptr; q.colptr = d.d_colptr; q.ve_slot = d.d_ve_slot; q.ve_chk = d.d_ve_chk;
-            q.syn_words = syn_words; q.err_words = err_words; q.conv = conv; q.iters = iters; q.ratio = ratio;
-            q.counters = counters;
+            common(q);
             q.off_syn = off_syn; q.off_resid = off_syn + h->SW * 4; q.off_dec = off_syn + 2 * h->SW * 4;
-            CU(h->variant == LDPCB200_VARIANT_MINSUM ? bp::single_launch_1(static_cast<int>(B), smem, st, q)
-               : h->variant == LDPCB200_VARIANT_FAST32 ? bp::single_launch_2(static_cast<int>(B), smem, st, q)
-                                                       : bp::single_launch_0(static_cast<int>(B), smem, st, q));
+            CU(K.single_launch(static_cast<int>(B), smem, st, q));
             h->launches++;
             return 0;
         }
@@ -1031,14 +1016,10 @@ int decode_on_device(ldpcb200 *h, DeviceCtx &d, int64_t B, const uint32_t *syn_w
             KernelTimer timer(h, d, st);
             if (h->dual) {
                 const int gl = static_cast<int>(std::min<long long>((groups + 1) / 2, static_cast<long long>(d.sm_count) * h->ctas_per_sm));
-                if (h->variant == LDPCB200_VARIANT_MINSUM) bp::smem_dual_launch_1(h->eb64, gl, 2 * thr, h->smem_bytes, st, q);
-                else if (h->variant == LDPCB200_VARIANT_FAST32) bp::smem_dual_launch_2(h->eb64, gl, 2 * thr, h->smem_bytes, st, q);
-                else bp::smem_dual_launch_0(h->eb64, gl, 2 * thr, h->smem_bytes, st, q);
+                K.dual_launch(h->eb64, gl, 2 * thr, h->smem_bytes, st, q);
             } else {
                 const int gl = static_cast<int>(std::min<long long>(groups, static_cast<long long>(d.sm_count) * h->ctas_per_sm));
-                if (h->variant == LDPCB200_VARIANT_MINSUM) bp::smem_kernel_launch_1(h->shape, h->eb64, gl, thr, h->smem_bytes, st, q);
-                else if (h->variant == LDPCB200_VARIANT_FAST32) bp::smem_kernel_launch_2(h->shape, h->eb64, gl, thr, h->smem_bytes, st, q);
-                else bp::smem_kernel_launch_0(h->shape, h->eb64, gl, thr, h->smem_bytes, st, q);
+                K.smem_launch(h->shape, h->eb64, gl, thr, h->smem_bytes, st, q);
             }
             h->launches++;
         }
@@ -1049,14 +1030,14 @@ int decode_on_device(ldpcb200 *h, DeviceCtx &d, int64_t B, const uint32_t *syn_w
             p.queue_ctr = f_count.as<unsigned int>() + 2;
         }
         KernelTimer timer(h, d, st);
-        kernel_launch_dispatch(h->variant, h->mode, h->big, h->shape, grid, thr, h->smem_bytes, st, p);
+        K.launch[h->mode][h->big](h->shape, grid, thr, h->smem_bytes, st, p);
         h->launches++;
     }
     CU(cudaGetLastError());
     return 0;
 }
 
-// ---- OSD-0 on the syndromes BP left unconverged (osd.cuh).  Stream-ordered; err_words is updated in place.
+// ---- OSD (osd.cuh)
 constexpr int kOsdThreads = 256;
 
 int osd_layout(const ldpcb200 *h, bp::OsdParams &p)
@@ -1078,23 +1059,27 @@ int osd_layout(const ldpcb200 *h, bp::OsdParams &p)
     return off > 0x7fffffffLL ? 0x7fffffff : static_cast<int>(off);
 }
 
-int osd0_on_device(ldpcb200 *h, DeviceCtx &d, DeviceCtx::StageSet &S, int64_t B, const uint32_t *syn_words,
-                   uint32_t *err_words, const uint8_t *conv, const double *ratio, unsigned long long *stats, cudaStream_t st)
+// OSD of order `order`, stream-ordered; err_words: BP decisions in, OSD result out.  Order 0 (OSD-0, osd0_kernel) runs
+// on the syndromes BP left unconverged, a higher order (osdk_kernel) on every syndrome of the batch.
+int osd_on_device(ldpcb200 *h, DeviceCtx &d, DeviceCtx::StageSet &S, int64_t B, int order, const uint32_t *syn_words,
+                  uint32_t *err_words, const uint8_t *conv, const double *ratio, unsigned long long *stats, cudaStream_t st)
 {
     if (B <= 0) return 0;
+    const char *what = order > 0 ? "OSD" : "OSD-0";
     if (h->variant != LDPCB200_VARIANT_EXACT)
-        return fail(LDPCB200_EUNSUPPORTED, "OSD-0 is defined on the posterior ratios of the exact variant");
-    if (B > 0x7fffffffLL) return fail(LDPCB200_EINVAL, "OSD-0: at most 2^31-1 syndromes per call");
-    if (h->s > static_cast<int64_t>(bp::kOsdMaxRowsPerThread) * kOsdThreads)
+        return fail(LDPCB200_EUNSUPPORTED, "%s is defined on the posterior ratios of the exact variant", what);
+    if (order < 0 || order > bp::kOsdMaxOrder) return fail(LDPCB200_EUNSUPPORTED, "osd_order must be between 0 and %d", bp::kOsdMaxOrder);
+    if (B > 0x7fffffffLL) return fail(LDPCB200_EINVAL, "%s: at most 2^31-1 syndromes per call", what);
+    if (order == 0 && h->s > static_cast<int64_t>(bp::kOsdMaxRowsPerThread) * kOsdThreads)
         return fail(LDPCB200_EUNSUPPORTED, "OSD-0: more than %d checks", bp::kOsdMaxRowsPerThread * kOsdThreads);
     CU(cudaSetDevice(d.device));
     bp::OsdParams p{};
     const int smem = osd_layout(h, p);
     if (smem > d.smem_optin)
-        return fail(LDPCB200_EUNSUPPORTED, "OSD-0: the bit-packed %lld x %lld matrix (%d bytes) does not fit in shared memory",
+        return fail(LDPCB200_EUNSUPPORTED, "%s: the bit-packed %lld x %lld matrix (%d bytes) does not fit in shared memory", what,
                     static_cast<long long>(h->s), static_cast<long long>(h->n), smem);
     int rc;
-    if ((rc = S.osd_list.reserve(static_cast<size_t>(B) * 4))) return rc;
+    if (order == 0 && (rc = S.osd_list.reserve(static_cast<size_t>(B) * 4))) return rc;
     if ((rc = S.osd_ctl.reserve(16))) return rc;
     if (!stats) {
         if ((rc = d.osd_stats.reserve(64))) return rc;
@@ -1103,64 +1088,46 @@ int osd0_on_device(ldpcb200 *h, DeviceCtx &d, DeviceCtx::StageSet &S, int64_t B,
     CU(cudaMemsetAsync(S.osd_ctl.p, 0, 16, st));
     p.colptr = d.d_colptr; p.rowval = d.d_ve_chk;
     p.syn_words = syn_words; p.err_words = err_words; p.ratio = ratio;
-    p.list = S.osd_list.as<int>(); p.count = S.osd_ctl.as<int>(); p.queue = S.osd_ctl.as<int>() + 1;
+    p.queue = S.osd_ctl.as<int>() + 1;
     p.stats = stats;
-    p.profile = h->opt_osd_profile;
-    bp::osd_collect_kernel<<<static_cast<unsigned>((B + 255) / 256), 256, 0, st>>>(conv, B, S.osd_list.as<int>(), S.osd_ctl.as<int>());
     const int per_sm = std::max(1, std::min(4, d.smem_per_sm / (smem + 1024)));
     const int grid = static_cast<int>(std::min<int64_t>(B, static_cast<int64_t>(d.sm_count) * per_sm));
-    auto launch = [&](auto kern) -> cudaError_t {
+    auto launch = [&](auto kern, auto... args) -> cudaError_t {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (e != cudaSuccess) return e;
-        kern<<<grid, kOsdThreads, smem, st>>>(p);
+        kern<<<grid, kOsdThreads, smem, st>>>(args...);
         return cudaSuccess;
     };
-    switch ((p.m + kOsdThreads - 1) / kOsdThreads) {
-        case 0: case 1: CU(launch(bp::osd0_kernel<kOsdThreads, 1>)); break;
-        case 2: CU(launch(bp::osd0_kernel<kOsdThreads, 2>)); break;
-        case 3: CU(launch(bp::osd0_kernel<kOsdThreads, 3>)); break;
-        case 4: CU(launch(bp::osd0_kernel<kOsdThreads, 4>)); break;
-        default: CU(launch(bp::osd0_kernel<kOsdThreads, 8>)); break;
+    if (order > 0) {
+        CU(launch(bp::osdk_kernel<kOsdThreads>, p, order, static_cast<long long>(B)));
+        h->launches++;
+    } else {
+        p.list = S.osd_list.as<int>(); p.count = S.osd_ctl.as<int>();
+        p.profile = h->opt_osd_profile;
+        bp::osd_collect_kernel<<<static_cast<unsigned>((B + 255) / 256), 256, 0, st>>>(conv, B, S.osd_list.as<int>(), S.osd_ctl.as<int>());
+        switch ((p.m + kOsdThreads - 1) / kOsdThreads) {
+            case 0: case 1: CU(launch(bp::osd0_kernel<kOsdThreads, 1>, p)); break;
+            case 2: CU(launch(bp::osd0_kernel<kOsdThreads, 2>, p)); break;
+            case 3: CU(launch(bp::osd0_kernel<kOsdThreads, 3>, p)); break;
+            case 4: CU(launch(bp::osd0_kernel<kOsdThreads, 4>, p)); break;
+            default: CU(launch(bp::osd0_kernel<kOsdThreads, 8>, p)); break;
+        }
+        h->launches += 2;
     }
-    h->launches += 2;
     CU(cudaGetLastError());
     return 0;
 }
 
-// ---- OSD of order O > 0 on EVERY syndrome of the batch (osd.cuh: osdk_kernel); err_words: BP decisions in, OSD result out.
-int osdk_on_device(ldpcb200 *h, DeviceCtx &d, DeviceCtx::StageSet &S, int64_t B, int order, const uint32_t *syn_words,
-                   uint32_t *err_words, const double *ratio, unsigned long long *stats, cudaStream_t st)
+// OSD of the handle's order after BP: where BP ran no iteration, log_probabs stays zero (reset!, belief_propagation.jl:86)
+// and the ratios are 1 everywhere.  Statistics go to d.osd_stats.
+int osd_after_bp(ldpcb200 *h, DeviceCtx &d, DeviceCtx::StageSet &S, int64_t B, const uint32_t *syn_words, uint32_t *err_words,
+                 const uint8_t *conv, double *ratio, cudaStream_t st)
 {
-    if (B <= 0) return 0;
-    if (h->variant != LDPCB200_VARIANT_EXACT)
-        return fail(LDPCB200_EUNSUPPORTED, "OSD is defined on the posterior ratios of the exact variant");
-    if (order < 1 || order > bp::kOsdMaxOrder) return fail(LDPCB200_EUNSUPPORTED, "osd_order must be between 0 and %d", bp::kOsdMaxOrder);
-    if (B > 0x7fffffffLL) return fail(LDPCB200_EINVAL, "OSD: at most 2^31-1 syndromes per call");
-    CU(cudaSetDevice(d.device));
-    bp::OsdParams p{};
-    const int smem = osd_layout(h, p);
-    if (smem > d.smem_optin)
-        return fail(LDPCB200_EUNSUPPORTED, "OSD: the bit-packed %lld x %lld matrix (%d bytes) does not fit in shared memory",
-                    static_cast<long long>(h->s), static_cast<long long>(h->n), smem);
-    int rc;
-    if ((rc = S.osd_ctl.reserve(16))) return rc;
-    if (!stats) {
-        if ((rc = d.osd_stats.reserve(64))) return rc;
-        stats = d.osd_stats.as<unsigned long long>();
+    if (h->max_iters <= 0) {
+        bp::osd_fill_ones_kernel<<<grid_for(B * h->n, d.sm_count), 256, 0, st>>>(ratio, B * h->n);
+        h->launches++;
     }
-    CU(cudaMemsetAsync(S.osd_ctl.p, 0, 16, st));
-    p.colptr = d.d_colptr; p.rowval = d.d_ve_chk;
-    p.syn_words = syn_words; p.err_words = err_words; p.ratio = ratio;
-    p.list = nullptr; p.count = nullptr; p.queue = S.osd_ctl.as<int>() + 1;
-    p.stats = stats;
-    const int per_sm = std::max(1, std::min(4, d.smem_per_sm / (smem + 1024)));
-    const int grid = static_cast<int>(std::min<int64_t>(B, static_cast<int64_t>(d.sm_count) * per_sm));
-    auto kern = bp::osdk_kernel<kOsdThreads>;
-    CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    kern<<<grid, kOsdThreads, smem, st>>>(p, order, B);
-    h->launches++;
-    CU(cudaGetLastError());
-    return 0;
+    return osd_on_device(h, d, S, B, h->opt_osd_order, syn_words, err_words, conv, ratio, d.osd_stats.as<unsigned long long>(), st);
 }
 
 // ---- BP-OTS (bpots.cuh): one CTA per syndrome.  Stream-ordered.
@@ -1243,7 +1210,37 @@ size_t fmt_bytes(int fmt, int64_t rows, int64_t ld, int64_t B, int RW)
     return 0;
 }
 
-inline int grid_for(long long work, int sm) { return static_cast<int>(std::max<long long>(1, std::min<long long>((work + 255) / 256, static_cast<long long>(sm) * 16))); }
+// Packed rows from B syndromes in the caller's format, already on the device at `raw` (U8 / I64: column stride ld).
+// PACKED32 needs no kernel: those rows are copied to syn_words as they are.
+void pack_syndromes(ldpcb200 *h, DeviceCtx &d, int fmt, const void *raw, int64_t ld, int64_t B, uint32_t *syn_words, cudaStream_t st)
+{
+    if (fmt == LDPCB200_FMT_PACKED32) return;
+    const int g = grid_for(B * h->SW, d.sm_count), s = static_cast<int>(h->s);
+    if (fmt == LDPCB200_FMT_BITS)
+        bp::pack_bits<<<g, 256, 0, st>>>(static_cast<const uint32_t *>(raw), (B * h->s + 31) / 32, s, h->SW, B, syn_words);
+    else if (fmt == LDPCB200_FMT_U8)
+        bp::pack_elems<uint8_t><<<g, 256, 0, st>>>(static_cast<const uint8_t *>(raw), ld, s, h->SW, B, syn_words);
+    else
+        bp::pack_elems<long long><<<g, 256, 0, st>>>(static_cast<const long long *>(raw), ld, s, h->SW, B, syn_words);
+    h->launches++;
+}
+
+// The caller's error format (BITS, U8, I64 or F64; column stride ld for the element formats) from B packed rows, on the device.
+void unpack_errors(ldpcb200 *h, DeviceCtx &d, int fmt, const uint32_t *err_words, int64_t B, void *raw, int64_t ld, cudaStream_t st)
+{
+    const int g = grid_for(B * h->NW, d.sm_count), n = static_cast<int>(h->n);
+    if (fmt == LDPCB200_FMT_BITS) {
+        const long long nw = (B * h->n + 31) / 32;
+        bp::unpack_bits<<<grid_for(nw, d.sm_count), 256, 0, st>>>(err_words, n, h->NW, B, static_cast<uint32_t *>(raw), nw);
+    } else if (fmt == LDPCB200_FMT_U8) {
+        bp::unpack_elems<uint8_t><<<g, 256, 0, st>>>(err_words, n, h->NW, B, static_cast<uint8_t *>(raw), ld);
+    } else if (fmt == LDPCB200_FMT_I64) {
+        bp::unpack_elems<long long><<<g, 256, 0, st>>>(err_words, n, h->NW, B, static_cast<long long *>(raw), ld);
+    } else {
+        bp::unpack_elems<double><<<g, 256, 0, st>>>(err_words, n, h->NW, B, static_cast<double *>(raw), ld);
+    }
+    h->launches++;
+}
 
 // Small host batch (decode! and a handful of columns): everything goes through ONE device block and its pinned
 // mirror -- one host->device copy, the kernels, one device->host copy, one synchronisation -- instead of the
@@ -1271,17 +1268,7 @@ int decode_host_tiny(ldpcb200 *h, DeviceCtx &d, int64_t B, const void *syndromes
     memcpy(P + o_in, syndromes, in_bytes);
     CU(cudaMemcpyAsync(in_packed ? static_cast<void *>(syn_words) : static_cast<void *>(D + o_in), P + o_in, in_bytes,
                        cudaMemcpyHostToDevice, st));
-    if (syn_fmt == LDPCB200_FMT_BITS)
-        bp::pack_bits<<<grid_for(B * h->SW, d.sm_count), 256, 0, st>>>(reinterpret_cast<uint32_t *>(D + o_in),
-                                                                       static_cast<long long>(in_bytes / 4), static_cast<int>(s), h->SW, B, syn_words);
-    else if (syn_fmt == LDPCB200_FMT_U8)
-        bp::pack_elems<uint8_t><<<grid_for(B * h->SW, d.sm_count), 256, 0, st>>>(D + o_in, syn_ld, static_cast<int>(s), h->SW, B, syn_words);
-    else if (syn_fmt == LDPCB200_FMT_I64)
-        bp::pack_elems<long long><<<grid_for(B * h->SW, d.sm_count), 256, 0, st>>>(reinterpret_cast<long long *>(D + o_in), syn_ld,
-                                                                                   static_cast<int>(s), h->SW, B, syn_words);
-    else if (!in_packed)
-        return fail(LDPCB200_EINVAL, "unsupported syndrome format %d", syn_fmt);
-    if (!in_packed) h->launches++;
+    pack_syndromes(h, d, syn_fmt, D + o_in, syn_ld, B, syn_words, st);
     // ---- decode
     CU(cudaMemsetAsync(D + o_out, 0, total - o_out, st));
     rc = decode_on_device(h, d, B, syn_words, err_words, D + o_conv, reinterpret_cast<int32_t *>(D + o_iters),
@@ -1289,25 +1276,8 @@ int decode_host_tiny(ldpcb200 *h, DeviceCtx &d, int64_t B, const void *syndromes
                           reinterpret_cast<unsigned long long *>(D + o_ctr), st);
     if (rc) return rc;
     // ---- out
-    const int g = grid_for(B * h->NW, d.sm_count);
-    if (err_fmt == LDPCB200_FMT_PACKED32) {
-        CU(cudaMemcpyAsync(D + o_out, err_words, errw_bytes, cudaMemcpyDeviceToDevice, st));
-    } else if (err_fmt == LDPCB200_FMT_BITS) {
-        bp::unpack_bits<<<grid_for(static_cast<long long>(out_bytes / 4), d.sm_count), 256, 0, st>>>(
-            err_words, static_cast<int>(n), h->NW, B, reinterpret_cast<uint32_t *>(D + o_out), static_cast<long long>(out_bytes / 4));
-        h->launches++;
-    } else if (err_fmt == LDPCB200_FMT_U8) {
-        bp::unpack_elems<uint8_t><<<g, 256, 0, st>>>(err_words, static_cast<int>(n), h->NW, B, D + o_out, err_ld);
-        h->launches++;
-    } else if (err_fmt == LDPCB200_FMT_I64) {
-        bp::unpack_elems<long long><<<g, 256, 0, st>>>(err_words, static_cast<int>(n), h->NW, B, reinterpret_cast<long long *>(D + o_out), err_ld);
-        h->launches++;
-    } else if (err_fmt == LDPCB200_FMT_F64) {
-        bp::unpack_elems<double><<<g, 256, 0, st>>>(err_words, static_cast<int>(n), h->NW, B, reinterpret_cast<double *>(D + o_out), err_ld);
-        h->launches++;
-    } else {
-        return fail(LDPCB200_EINVAL, "unsupported error format %d", err_fmt);
-    }
+    if (err_fmt == LDPCB200_FMT_PACKED32) CU(cudaMemcpyAsync(D + o_out, err_words, errw_bytes, cudaMemcpyDeviceToDevice, st));
+    else unpack_errors(h, d, err_fmt, err_words, B, D + o_out, err_ld, st);
     CU(cudaMemcpyAsync(P + o_out, D + o_out, total - o_out, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     const bool elems = err_fmt == LDPCB200_FMT_U8 || err_fmt == LDPCB200_FMT_I64 || err_fmt == LDPCB200_FMT_F64;
@@ -1457,30 +1427,14 @@ int decode_host_range(ldpcb200 *h, DeviceCtx &d, int64_t b0, int64_t Bd, int64_t
         uint32_t *syn_words = S.syn_words.as<uint32_t>();
         if (syn_fmt == LDPCB200_FMT_PACKED32) {
             if ((rc = h2d(syn_words, static_cast<const uint32_t *>(syndromes) + g0 * h->SW, static_cast<size_t>(Bc) * h->SW * 4, pg_in))) return rc;
-        } else if (syn_fmt == LDPCB200_FMT_BITS) {
-            const size_t w0 = static_cast<size_t>(g0 * s / 32);           // g0 is a multiple of 32
-            const size_t nw = static_cast<size_t>((Bc * s + 31) / 32);
-            if ((rc = S.raw_in.reserve(nw * 4))) return rc;
-            if ((rc = h2d(S.raw_in.p, static_cast<const uint32_t *>(syndromes) + w0, nw * 4, pg_in))) return rc;
-            bp::pack_bits<<<grid_for(Bc * h->SW, d.sm_count), 256, 0, st>>>(S.raw_in.as<uint32_t>(), static_cast<long long>(nw),
-                                                                            static_cast<int>(s), h->SW, Bc, syn_words);
-            h->launches++;
-        } else if (syn_fmt == LDPCB200_FMT_U8) {
-            const size_t bytes = fmt_bytes(syn_fmt, s, syn_ld, Bc, h->SW);
-            if ((rc = S.raw_in.reserve(bytes))) return rc;
-            if ((rc = h2d(S.raw_in.p, static_cast<const uint8_t *>(syndromes) + g0 * syn_ld, bytes, pg_in))) return rc;
-            bp::pack_elems<uint8_t><<<grid_for(Bc * h->SW, d.sm_count), 256, 0, st>>>(S.raw_in.as<uint8_t>(), syn_ld,
-                                                                                     static_cast<int>(s), h->SW, Bc, syn_words);
-            h->launches++;
-        } else if (syn_fmt == LDPCB200_FMT_I64) {
-            const size_t bytes = fmt_bytes(syn_fmt, s, syn_ld, Bc, h->SW);
-            if ((rc = S.raw_in.reserve(bytes))) return rc;
-            if ((rc = h2d(S.raw_in.p, static_cast<const long long *>(syndromes) + g0 * syn_ld, bytes, pg_in))) return rc;
-            bp::pack_elems<long long><<<grid_for(Bc * h->SW, d.sm_count), 256, 0, st>>>(S.raw_in.as<long long>(), syn_ld,
-                                                                                       static_cast<int>(s), h->SW, Bc, syn_words);
-            h->launches++;
         } else {
-            return fail(LDPCB200_EINVAL, "unsupported syndrome format %d", syn_fmt);
+            // column g0 of the caller's buffer (g0 is a multiple of 32: whole words of the bit stream)
+            const size_t at = syn_fmt == LDPCB200_FMT_BITS ? static_cast<size_t>(g0 * s / 8)
+                                                           : static_cast<size_t>(g0 * syn_ld) * (syn_fmt == LDPCB200_FMT_I64 ? 8 : 1);
+            const size_t bytes = fmt_bytes(syn_fmt, s, syn_ld, Bc, h->SW);
+            if ((rc = S.raw_in.reserve(bytes))) return rc;
+            if ((rc = h2d(S.raw_in.p, static_cast<const uint8_t *>(syndromes) + at, bytes, pg_in))) return rc;
+            pack_syndromes(h, d, syn_fmt, S.raw_in.p, syn_ld, Bc, syn_words, st);
         }
         // BitMatrix output: the shared-memory kernel writes the caller's bit stream itself (no conversion kernel between the
         // decode and the copy out)
@@ -1512,56 +1466,26 @@ int decode_host_range(ldpcb200 *h, DeviceCtx &d, int64_t b0, int64_t Bd, int64_t
         if (rc) return rc;
         CU(cudaEventRecord(d.decode_done, st));
         have_prev_decode = true;
-        if (osd) {
-            if (h->max_iters <= 0) {          // log_probabs stays zero (reset!, belief_propagation.jl:86): ratio 1 everywhere
-                bp::osd_fill_ones_kernel<<<grid_for(Bc * n, d.sm_count), 256, 0, st>>>(S.ratio.as<double>(), Bc * n);
-                h->launches++;
-            }
-            if (h->opt_osd_order > 0)
-                rc = osdk_on_device(h, d, S, Bc, h->opt_osd_order, syn_words, S.err_words.as<uint32_t>(), S.ratio.as<double>(),
-                                    d.osd_stats.as<unsigned long long>(), st);
-            else
-                rc = osd0_on_device(h, d, S, Bc, syn_words, S.err_words.as<uint32_t>(), S.conv.as<uint8_t>(), S.ratio.as<double>(),
-                                    d.osd_stats.as<unsigned long long>(), st);
-            if (rc) return rc;
-        }
+        if (osd && (rc = osd_after_bp(h, d, S, Bc, syn_words, S.err_words.as<uint32_t>(), S.conv.as<uint8_t>(), S.ratio.as<double>(), st)))
+            return rc;
         // ---- packed rows -> caller's format -> host
-        const uint32_t *ew = S.err_words.as<uint32_t>();
         if (err_fmt == LDPCB200_FMT_PACKED32) {
-            if ((rc = d2h(static_cast<uint32_t *>(errors) + g0 * h->NW, ew, static_cast<size_t>(Bc) * h->NW * 4, pg_out))) return rc;
-        } else if (err_fmt == LDPCB200_FMT_BITS) {
-            const size_t w0 = static_cast<size_t>(g0 * n / 32);
-            const size_t nw = static_cast<size_t>((Bc * n + 31) / 32);
-            if ((rc = S.raw_out.reserve(nw * 4))) return rc;
-            if (!bits_done) {
-                bp::unpack_bits<<<grid_for(static_cast<long long>(nw), d.sm_count), 256, 0, st>>>(
-                    ew, static_cast<int>(n), h->NW, Bc, S.raw_out.as<uint32_t>(), static_cast<long long>(nw));
-                h->launches++;
-            }
+            if ((rc = d2h(static_cast<uint32_t *>(errors) + g0 * h->NW, S.err_words.p, static_cast<size_t>(Bc) * h->NW * 4, pg_out))) return rc;
+        } else {
+            const bool bits = err_fmt == LDPCB200_FMT_BITS;
+            const size_t bytes = fmt_bytes(err_fmt, n, err_ld, Bc, h->NW), esz = err_fmt == LDPCB200_FMT_U8 ? 1 : 8;
+            // column g0 of the caller's buffer (g0 is a multiple of 32: whole words of the bit stream)
+            uint8_t *dst = static_cast<uint8_t *>(errors) + (bits ? static_cast<size_t>(g0 * n / 8) : static_cast<size_t>(g0) * err_ld * esz);
+            if ((rc = S.raw_out.reserve(bytes))) return rc;
+            if (!bits && err_ld != n) CU(cudaMemsetAsync(S.raw_out.p, 0, bytes, st));
+            if (!bits_done) unpack_errors(h, d, err_fmt, S.err_words.as<uint32_t>(), Bc, S.raw_out.p, err_ld, st);
             // (the last word of a chunk may hold bits of the next chunk's first column only when Bc*n is not a multiple
             //  of 32, i.e. in the final chunk of the batch: chunk boundaries are multiples of 32 columns)
-            if ((rc = d2h(static_cast<uint32_t *>(errors) + w0, S.raw_out.p, nw * 4, pg_out))) return rc;
-        } else if (err_fmt == LDPCB200_FMT_U8 || err_fmt == LDPCB200_FMT_I64 || err_fmt == LDPCB200_FMT_F64) {
-            const size_t bytes = fmt_bytes(err_fmt, n, err_ld, Bc, h->NW);
-            if ((rc = S.raw_out.reserve(bytes))) return rc;
-            const int g = grid_for(Bc * h->NW, d.sm_count);
-            if (err_ld != n) CU(cudaMemsetAsync(S.raw_out.p, 0, bytes, st));
-            if (err_fmt == LDPCB200_FMT_U8)
-                bp::unpack_elems<uint8_t><<<g, 256, 0, st>>>(ew, static_cast<int>(n), h->NW, Bc, S.raw_out.as<uint8_t>(), err_ld);
-            else if (err_fmt == LDPCB200_FMT_I64)
-                bp::unpack_elems<long long><<<g, 256, 0, st>>>(ew, static_cast<int>(n), h->NW, Bc, S.raw_out.as<long long>(), err_ld);
-            else
-                bp::unpack_elems<double><<<g, 256, 0, st>>>(ew, static_cast<int>(n), h->NW, Bc, S.raw_out.as<double>(), err_ld);
-            h->launches++;
-            const size_t esz = err_fmt == LDPCB200_FMT_U8 ? 1 : 8;
-            if (err_ld == n) {
-                if ((rc = d2h(static_cast<uint8_t *>(errors) + static_cast<size_t>(g0) * err_ld * esz, S.raw_out.p, bytes, pg_out))) return rc;
+            if (bits || err_ld == n) {
+                if ((rc = d2h(dst, S.raw_out.p, bytes, pg_out))) return rc;
             } else {   // strided destination: only the n rows of each column belong to the caller
-                CU(cudaMemcpy2DAsync(static_cast<uint8_t *>(errors) + static_cast<size_t>(g0) * err_ld * esz, err_ld * esz,
-                                     S.raw_out.p, err_ld * esz, n * esz, Bc, cudaMemcpyDeviceToHost, st));
+                CU(cudaMemcpy2DAsync(dst, err_ld * esz, S.raw_out.p, err_ld * esz, n * esz, Bc, cudaMemcpyDeviceToHost, st));
             }
-        } else {
-            return fail(LDPCB200_EINVAL, "unsupported error format %d", err_fmt);
         }
         if ((rc = d2h(converged + g0, S.conv.p, static_cast<size_t>(Bc), pg_conv))) return rc;
         if (iters && (rc = d2h(iters + g0, S.iters.p, static_cast<size_t>(Bc) * 4, pg_iters))) return rc;
@@ -1641,9 +1565,55 @@ int nccl_sum_block(ldpcb200 *h, int count, Src src, int64_t *out)
     for (int c = 0; c < count; ++c) out[c] = static_cast<int64_t>(hc[c]);
     return 0;
 }
-int nccl_sum_counters(ldpcb200 *h, int64_t *out)
+
+// Per-device blocks of `count` values each, added on the host into out
+void host_sum(const std::vector<int64_t> &per_dev, int count, int64_t *out)
 {
-    return nccl_sum_block(h, LDPCB200_NUM_COUNTERS, [](DeviceCtx &d) { return d.counters.p; }, out);
+    for (size_t i = 0; i < per_dev.size(); ++i) out[i % count] += per_dev[i];
+}
+
+// Split `total` columns into contiguous per-device ranges, boundaries multiples of 32 (bit formats stay word aligned),
+// and run work(k, first, count) for every device k: inline for one device, on one thread per device otherwise.
+// Returns the first failing device's code, with its message.
+template <class Work>
+int fan_out(ldpcb200 *h, int64_t total, Work work)
+{
+    const int nd = static_cast<int>(h->dev.size());
+    std::vector<int64_t> lo(nd + 1, 0);
+    const int64_t blocks = (total + 31) / 32;
+    for (int k = 0; k <= nd; ++k) lo[k] = std::min<int64_t>(total, (blocks * k / nd) * 32);
+    lo[nd] = total;
+    std::vector<int> rcs(nd, 0);
+    std::vector<std::string> errs(nd);
+    auto run = [&](int k) {
+        rcs[k] = work(k, lo[k], lo[k + 1] - lo[k]);
+        if (rcs[k]) errs[k] = g_err;
+    };
+    if (nd == 1) {
+        run(0);
+    } else {
+        std::vector<std::thread> th;
+        for (int k = 0; k < nd; ++k) th.emplace_back(run, k);
+        for (auto &t : th) t.join();
+    }
+    for (int k = 0; k < nd; ++k)
+        if (rcs[k]) { g_err = errs[k]; return rcs[k]; }
+    return 0;
+}
+
+// B error rows with independent flips of probability per (rows first .. first+B-1 of the stream `seed`) and their syndromes,
+// as packed rows on the device
+int sample_on_device(ldpcb200 *h, DeviceCtx &d, int64_t B, int64_t first, uint64_t seed, double per, uint32_t *err_words,
+                     uint32_t *syn_words, cudaStream_t st)
+{
+    const double t = std::floor(per * 4294967296.0);
+    const uint32_t thr = !(t > 0) ? 0u : (t >= 4294967295.0 ? 0xFFFFFFFFu : static_cast<uint32_t>(t));
+    CU(cudaMemsetAsync(syn_words, 0, static_cast<size_t>(B) * h->SW * 4, st));
+    bp::sample_errors<<<grid_for(B * h->NW, d.sm_count), 256, 0, st>>>(static_cast<int>(h->n), h->NW, B, first, static_cast<uint32_t>(seed),
+                                                                      static_cast<uint32_t>(seed >> 32), thr, err_words);
+    bp::syndrome_of<<<grid_for(B * h->NW, d.sm_count), 256, 0, st>>>(d.d_colptr, d.d_ve_chk, h->NW, h->SW, B, err_words, syn_words);
+    h->launches += 2;
+    return 0;
 }
 
 // One device's share of the sampling + scoring harness: tiles of device-resident shots.
@@ -1673,18 +1643,11 @@ int harness_on_device(ldpcb200 *h, DeviceCtx &d, int64_t first, int64_t shots, u
             if ((rc = d.lmask.reserve(h->lmask.size() * 8))) return rc;
             CU(cudaMemcpyAsync(d.lmask.p, h->lmask.data(), h->lmask.size() * 8, cudaMemcpyHostToDevice, st));
         }
-        double t = std::floor(per_channel * 4294967296.0);
-        const uint32_t thr = !(t > 0) ? 0u : (t >= 4294967295.0 ? 0xFFFFFFFFu : static_cast<uint32_t>(t));
         unsigned long long *ctr = d.hs_ctr.as<unsigned long long>();
         for (int64_t t0 = 0; t0 < shots; t0 += tile) {
             const int64_t bt = std::min(tile, shots - t0);
-            CU(cudaMemsetAsync(d.hs_syn.p, 0, static_cast<size_t>(bt) * h->SW * 4, st));
-            bp::sample_errors<<<grid_for(bt * h->NW, d.sm_count), 256, 0, st>>>(static_cast<int>(h->n), h->NW, bt, first + t0,
-                                                                               static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32), thr,
-                                                                               d.hs_truth.as<uint32_t>());
-            bp::syndrome_of<<<grid_for(bt * h->NW, d.sm_count), 256, 0, st>>>(d.d_colptr, d.d_ve_chk, h->NW, h->SW, bt, d.hs_truth.as<uint32_t>(),
-                                                                             d.hs_syn.as<uint32_t>());
-            h->launches += 2;
+            if ((rc = sample_on_device(h, d, bt, first + t0, seed, per_channel, d.hs_truth.as<uint32_t>(), d.hs_syn.as<uint32_t>(), st)))
+                return rc;
             const bool want_ratio = osd && h->max_iters > 0;
             if (ots)
                 rc = bpots_on_device(h, d, bt, d.hs_syn.as<uint32_t>(), d.hs_err.as<uint32_t>(), d.hs_conv.as<uint8_t>(), d.hs_iters.as<int32_t>(),
@@ -1693,19 +1656,9 @@ int harness_on_device(ldpcb200 *h, DeviceCtx &d, int64_t first, int64_t shots, u
                 rc = decode_on_device(h, d, bt, d.hs_syn.as<uint32_t>(), d.hs_err.as<uint32_t>(), d.hs_conv.as<uint8_t>(), d.hs_iters.as<int32_t>(),
                                       want_ratio ? d.hs_ratio.as<double>() : nullptr, ctr + LDPCB200_NUM_HARNESS_COUNTERS, st, h->opt_osd_order == 0);
             if (rc) return rc;
-            if (osd) {
-                if (h->max_iters <= 0) {
-                    bp::osd_fill_ones_kernel<<<grid_for(bt * h->n, d.sm_count), 256, 0, st>>>(d.hs_ratio.as<double>(), bt * h->n);
-                    h->launches++;
-                }
-                if (h->opt_osd_order > 0)
-                    rc = osdk_on_device(h, d, d.set[0], bt, h->opt_osd_order, d.hs_syn.as<uint32_t>(), d.hs_err.as<uint32_t>(),
-                                        d.hs_ratio.as<double>(), d.osd_stats.as<unsigned long long>(), st);
-                else
-                    rc = osd0_on_device(h, d, d.set[0], bt, d.hs_syn.as<uint32_t>(), d.hs_err.as<uint32_t>(), d.hs_conv.as<uint8_t>(),
-                                        d.hs_ratio.as<double>(), d.osd_stats.as<unsigned long long>(), st);
-                if (rc) return rc;
-            }
+            if (osd && (rc = osd_after_bp(h, d, d.set[0], bt, d.hs_syn.as<uint32_t>(), d.hs_err.as<uint32_t>(), d.hs_conv.as<uint8_t>(),
+                                          d.hs_ratio.as<double>(), st)))
+                return rc;
             bp::score_rows_logical<<<grid_for(bt * 32, d.sm_count), 256, 0, st>>>(
                 d.d_colptr, d.d_ve_chk, h->NW, h->SW, bt, d.hs_truth.as<uint32_t>(), d.hs_err.as<uint32_t>(), d.hs_syn.as<uint32_t>(),
                 d.scratch.as<uint32_t>(), h->lmask.empty() ? nullptr : d.lmask.as<unsigned long long>(), ctr + 3);
@@ -1719,6 +1672,16 @@ int harness_on_device(ldpcb200 *h, DeviceCtx &d, int64_t first, int64_t shots, u
     CU(cudaMemcpyAsync(hc, d.hs_ctr.p, sizeof(hc), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     for (int k = 0; k < LDPCB200_NUM_HARNESS_COUNTERS; ++k) out8[k] = static_cast<int64_t>(hc[k]);
+    return 0;
+}
+
+// The device of a call on device-resident buffers, and its stream: the caller's, or the device's own when that is null
+int device_of(ldpcb200 *h, int32_t dev_slot, void *stream, DeviceCtx *&d, cudaStream_t &st)
+{
+    if (!h) return fail(LDPCB200_EINVAL, "null handle");
+    if (dev_slot < 0 || dev_slot >= static_cast<int>(h->dev.size())) return fail(LDPCB200_EINVAL, "bad dev_slot");
+    d = &h->dev[dev_slot];
+    st = stream ? static_cast<cudaStream_t>(stream) : d->stream;
     return 0;
 }
 
@@ -1764,19 +1727,8 @@ int ldpcb200_create(int64_t s, int64_t n, const int64_t *colptr, const int64_t *
         return fail(LDPCB200_ENODEVICE, "no CUDA device available (%s); libldpcb200 has no CPU fallback",
                     e != cudaSuccess ? cudaGetErrorString(e) : "device count 0");
     ldpcb200 *h = new ldpcb200();
-    h->s = s; h->n = n; h->per = per; h->max_iters = max_iters; h->variant = variant;
-    // channel_probs[j] / (1 - channel_probs[j]) (belief_propagation.jl:129,153), IEEE double on the host
-    {
-        volatile double one_minus = 1.0 - per;
-        volatile double q = per / one_minus;
-        h->p0 = q;
-        h->regular_p0 = std::isnormal(h->p0) && h->p0 > 0.0;
-        if (variant != LDPCB200_VARIANT_EXACT) {        // the kernels' prior slot carries L0 = log((1-p)/p)
-            volatile double r = one_minus / per;
-            h->p0 = std::log(r);
-            if (variant == LDPCB200_VARIANT_FAST32) h->p0 = static_cast<double>(static_cast<float>(h->p0));
-        }
-    }
+    h->s = s; h->n = n; h->max_iters = max_iters; h->variant = variant;
+    set_prior(h, per);
     int rc = build_graph(h, colptr, rowval, index_base);
     if (rc) { delete h; return rc; }
     if (variant != LDPCB200_VARIANT_EXACT && h->big) {
@@ -1886,14 +1838,14 @@ int ldpcb200_decode_device(ldpcb200_t *h, int32_t dev_slot, int64_t B, const uin
                            uint8_t *d_converged, int32_t *d_iters, double *d_posterior_ratio,
                            unsigned long long *d_counters, void *stream)
 {
-    if (!h) return fail(LDPCB200_EINVAL, "null handle");
-    if (dev_slot < 0 || dev_slot >= static_cast<int>(h->dev.size())) return fail(LDPCB200_EINVAL, "bad dev_slot");
-    if (B < 0 || (B > 0 && (!d_syn_words || !d_err_words || !d_converged))) return fail(LDPCB200_EINVAL, "null device buffer");
-    int rc = configure(h);
+    DeviceCtx *d;
+    cudaStream_t st;
+    int rc = device_of(h, dev_slot, stream, d, st);
     if (rc) return rc;
-    DeviceCtx &d = h->dev[dev_slot];
-    return decode_on_device(h, d, B, d_syn_words, d_err_words, d_converged, d_iters, d_posterior_ratio, d_counters,
-                            stream ? static_cast<cudaStream_t>(stream) : d.stream, h->opt_ratio_last_only != 0);
+    if (B < 0 || (B > 0 && (!d_syn_words || !d_err_words || !d_converged))) return fail(LDPCB200_EINVAL, "null device buffer");
+    if ((rc = configure(h))) return rc;
+    return decode_on_device(h, *d, B, d_syn_words, d_err_words, d_converged, d_iters, d_posterior_ratio, d_counters, st,
+                            h->opt_ratio_last_only != 0);
 }
 
 static int decode_batch_impl(ldpcb200_t *h, int64_t B, const void *syndromes, int32_t syn_fmt, int64_t syn_ld, void *errors,
@@ -1909,58 +1861,33 @@ static int decode_batch_impl(ldpcb200_t *h, int64_t B, const void *syndromes, in
     if (B == 0) return 0;
     if (!syndromes || !errors || !converged) return fail(LDPCB200_EINVAL, "null host buffer");
     if (syn_fmt == LDPCB200_FMT_F64) return fail(LDPCB200_EINVAL, "FMT_F64 is an output-only format");
+    if (syn_fmt < LDPCB200_FMT_U8 || syn_fmt > LDPCB200_FMT_PACKED32) return fail(LDPCB200_EINVAL, "unsupported syndrome format %d", syn_fmt);
+    if (err_fmt < LDPCB200_FMT_U8 || err_fmt > LDPCB200_FMT_F64) return fail(LDPCB200_EINVAL, "unsupported error format %d", err_fmt);
     if ((syn_fmt == LDPCB200_FMT_U8 || syn_fmt == LDPCB200_FMT_I64) && syn_ld < h->s) return fail(LDPCB200_EINVAL, "syn_ld < s");
     if ((err_fmt == LDPCB200_FMT_U8 || err_fmt == LDPCB200_FMT_I64 || err_fmt == LDPCB200_FMT_F64) && err_ld < h->n)
         return fail(LDPCB200_EINVAL, "err_ld < n");
     int rc = configure(h);
     if (rc) return rc;
     const int nd = static_cast<int>(h->dev.size());
-    // contiguous column ranges per device, boundaries multiples of 32 (bit formats stay word aligned)
-    std::vector<int64_t> lo(nd + 1, 0);
-    const int64_t blocks = (B + 31) / 32;
-    for (int k = 0; k <= nd; ++k) lo[k] = std::min<int64_t>(B, (blocks * k / nd) * 32);
-    lo[nd] = B;
-    std::vector<int> rcs(nd, 0);
-    std::vector<std::string> errs(nd);
     std::vector<int64_t> ctr(static_cast<size_t>(nd) * LDPCB200_NUM_COUNTERS, 0);
     std::vector<int64_t> ost(static_cast<size_t>(nd) * LDPCB200_NUM_OSD_STATS, 0);
-    auto work = [&](int k) {
-        if (lo[k + 1] > lo[k])
-            rcs[k] = decode_host_range(h, h->dev[k], lo[k], lo[k + 1] - lo[k], B, syndromes, syn_fmt, syn_ld, errors, err_fmt,
-                                       err_ld, converged, iters, posterior_ratio, &ctr[static_cast<size_t>(k) * LDPCB200_NUM_COUNTERS],
-                                       osd, &ost[static_cast<size_t>(k) * LDPCB200_NUM_OSD_STATS], ots);
-        if (rcs[k]) errs[k] = g_err;
-    };
-    if (nd == 1) {
-        work(0);
-    } else {
-        std::vector<std::thread> th;
-        for (int k = 0; k < nd; ++k) th.emplace_back(work, k);
-        for (auto &t : th) t.join();
-    }
-    for (int k = 0; k < nd; ++k)
-        if (rcs[k]) { g_err = errs[k]; return rcs[k]; }
+    rc = fan_out(h, B, [&](int k, int64_t b0, int64_t Bd) {
+        return Bd <= 0 ? 0 : decode_host_range(h, h->dev[k], b0, Bd, B, syndromes, syn_fmt, syn_ld, errors, err_fmt, err_ld, converged,
+                                               iters, posterior_ratio, &ctr[static_cast<size_t>(k) * LDPCB200_NUM_COUNTERS], osd,
+                                               &ost[static_cast<size_t>(k) * LDPCB200_NUM_OSD_STATS], ots);
+    });
+    if (rc) return rc;
     if (counters) {
-        bool summed = false;
-        if (nd > 1) {
-            nccl_prepare(h);
-            // every device must have decoded a share (its counter block then holds this call's values; a batch too
-            // small for that is summed on the host)
-            bool all_shares = true;
-            for (int k = 0; k < nd; ++k) all_shares &= lo[k + 1] > lo[k];
-            if (h->nccl_state == 1 && all_shares) {
-                int rc2 = nccl_sum_counters(h, counters);
-                if (rc2) return rc2;
-                summed = true;
-            }
+        if (nd > 1) nccl_prepare(h);
+        // NCCL only when every device decoded a share -- fan_out gives each one 32 columns or more when there are at least
+        // nd blocks of 32 -- so that its counter block holds this call's values; a smaller batch is summed on the host
+        if (h->nccl_state == 1 && (B + 31) / 32 >= nd) {
+            if ((rc = nccl_sum_block(h, LDPCB200_NUM_COUNTERS, [](DeviceCtx &d) { return d.counters.p; }, counters))) return rc;
+        } else {
+            host_sum(ctr, LDPCB200_NUM_COUNTERS, counters);
         }
-        if (!summed)
-            for (int k = 0; k < nd; ++k)
-                for (int c = 0; c < LDPCB200_NUM_COUNTERS; ++c) counters[c] += ctr[static_cast<size_t>(k) * LDPCB200_NUM_COUNTERS + c];
     }
-    if (osd_stats)
-        for (int k = 0; k < nd; ++k)
-            for (int c = 0; c < LDPCB200_NUM_OSD_STATS; ++c) osd_stats[c] += ost[static_cast<size_t>(k) * LDPCB200_NUM_OSD_STATS + c];
+    if (osd_stats) host_sum(ost, LDPCB200_NUM_OSD_STATS, osd_stats);
     return 0;
 }
 
@@ -1990,45 +1917,38 @@ int ldpcb200_bpots_decode_batch(ldpcb200_t *h, int64_t B, const void *syndromes,
 int ldpcb200_bpots_device(ldpcb200_t *h, int32_t dev_slot, int64_t B, const uint32_t *d_syn_words, uint32_t *d_err_words,
                           uint8_t *d_converged, int32_t *d_iters, unsigned long long *d_counters, int32_t T, double C, void *stream)
 {
-    if (!h) return fail(LDPCB200_EINVAL, "null handle");
-    if (dev_slot < 0 || dev_slot >= static_cast<int>(h->dev.size())) return fail(LDPCB200_EINVAL, "bad dev_slot");
+    DeviceCtx *d;
+    cudaStream_t st;
+    int rc = device_of(h, dev_slot, stream, d, st);
+    if (rc) return rc;
     if (B < 0 || (B > 0 && (!d_syn_words || !d_err_words || !d_converged))) return fail(LDPCB200_EINVAL, "null device buffer");
-    DeviceCtx &d = h->dev[dev_slot];
     const BpotsArgs a{T, C};
-    return bpots_on_device(h, d, B, d_syn_words, d_err_words, d_converged, d_iters, a, d_counters,
-                           stream ? static_cast<cudaStream_t>(stream) : d.stream);
+    return bpots_on_device(h, *d, B, d_syn_words, d_err_words, d_converged, d_iters, a, d_counters, st);
 }
 
 int ldpcb200_osd0_device(ldpcb200_t *h, int32_t dev_slot, int64_t B, const uint32_t *d_syn_words, uint32_t *d_err_words,
                          const uint8_t *d_converged, const double *d_posterior_ratio, unsigned long long *d_stats, void *stream)
 {
-    if (!h) return fail(LDPCB200_EINVAL, "null handle");
-    if (dev_slot < 0 || dev_slot >= static_cast<int>(h->dev.size())) return fail(LDPCB200_EINVAL, "bad dev_slot");
+    DeviceCtx *d;
+    cudaStream_t st;
+    int rc = device_of(h, dev_slot, stream, d, st);
+    if (rc) return rc;
     if (B < 0 || (B > 0 && (!d_syn_words || !d_err_words || !d_converged || !d_posterior_ratio)))
         return fail(LDPCB200_EINVAL, "null device buffer");
-    DeviceCtx &d = h->dev[dev_slot];
-    return osd0_on_device(h, d, d.set[0], B, d_syn_words, d_err_words, d_converged, d_posterior_ratio, d_stats,
-                          stream ? static_cast<cudaStream_t>(stream) : d.stream);
+    return osd_on_device(h, *d, d->set[0], B, 0, d_syn_words, d_err_words, d_converged, d_posterior_ratio, d_stats, st);
 }
 
 int ldpcb200_sample_device(ldpcb200_t *h, int32_t dev_slot, int64_t B, int64_t first, uint64_t seed, double per,
                            uint32_t *d_true_err_words, uint32_t *d_syn_words, void *stream)
 {
-    if (!h || dev_slot < 0 || dev_slot >= static_cast<int>(h->dev.size())) return fail(LDPCB200_EINVAL, "bad handle / dev_slot");
+    DeviceCtx *d;
+    cudaStream_t st;
+    int rc = device_of(h, dev_slot, stream, d, st);
+    if (rc) return rc;
     if (B <= 0) return 0;
     if (!d_true_err_words || !d_syn_words) return fail(LDPCB200_EINVAL, "null device buffer");
-    DeviceCtx &d = h->dev[dev_slot];
-    CU(cudaSetDevice(d.device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d.stream;
-    double t = std::floor(per * 4294967296.0);
-    uint32_t thr = !(t > 0) ? 0u : (t >= 4294967295.0 ? 0xFFFFFFFFu : static_cast<uint32_t>(t));
-    CU(cudaMemsetAsync(d_syn_words, 0, static_cast<size_t>(B) * h->SW * 4, st));
-    bp::sample_errors<<<grid_for(B * h->NW, d.sm_count), 256, 0, st>>>(static_cast<int>(h->n), h->NW, B, first,
-                                                                      static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32),
-                                                                      thr, d_true_err_words);
-    bp::syndrome_of<<<grid_for(B * h->NW, d.sm_count), 256, 0, st>>>(d.d_colptr, d.d_ve_chk, h->NW, h->SW, B, d_true_err_words,
-                                                                    d_syn_words);
-    h->launches += 2;
+    CU(cudaSetDevice(d->device));
+    if ((rc = sample_on_device(h, *d, B, first, seed, per, d_true_err_words, d_syn_words, st))) return rc;
     CU(cudaGetLastError());
     return 0;
 }
@@ -2036,17 +1956,17 @@ int ldpcb200_sample_device(ldpcb200_t *h, int32_t dev_slot, int64_t B, int64_t f
 int ldpcb200_score_device(ldpcb200_t *h, int32_t dev_slot, int64_t B, const uint32_t *d_true_err_words,
                           const uint32_t *d_err_words, const uint32_t *d_syn_words, unsigned long long *d_out, void *stream)
 {
-    if (!h || dev_slot < 0 || dev_slot >= static_cast<int>(h->dev.size())) return fail(LDPCB200_EINVAL, "bad handle / dev_slot");
+    DeviceCtx *d;
+    cudaStream_t st;
+    int rc = device_of(h, dev_slot, stream, d, st);
+    if (rc) return rc;
     if (B <= 0) return 0;
     if (!d_true_err_words || !d_err_words || !d_syn_words || !d_out) return fail(LDPCB200_EINVAL, "null device buffer");
-    DeviceCtx &d = h->dev[dev_slot];
-    CU(cudaSetDevice(d.device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d.stream;
-    int rc = d.scratch.reserve(static_cast<size_t>(B) * h->SW * 4);
-    if (rc) return rc;
-    bp::score_rows<<<grid_for(B * 32, d.sm_count), 256, 0, st>>>(d.d_rowptr, d.d_colptr, d.d_ve_chk, h->NW, h->SW, B,
-                                                                d_true_err_words, d_err_words, d_syn_words,
-                                                                d.scratch.as<uint32_t>(), d_out);
+    CU(cudaSetDevice(d->device));
+    if ((rc = d->scratch.reserve(static_cast<size_t>(B) * h->SW * 4))) return rc;
+    bp::score_rows<<<grid_for(B * 32, d->sm_count), 256, 0, st>>>(d->d_rowptr, d->d_colptr, d->d_ve_chk, h->NW, h->SW, B,
+                                                                 d_true_err_words, d_err_words, d_syn_words,
+                                                                 d->scratch.as<uint32_t>(), d_out);
     h->launches++;
     CU(cudaGetLastError());
     return 0;
@@ -2085,17 +2005,17 @@ int ldpcb200_set_logicals(ldpcb200_t *h, int64_t k, const int64_t *colptr, const
 int ldpcb200_score_logical_device(ldpcb200_t *h, int32_t dev_slot, int64_t B, const uint32_t *d_true_err_words,
                                   const uint32_t *d_err_words, const uint32_t *d_syn_words, unsigned long long *d_out, void *stream)
 {
-    if (!h || dev_slot < 0 || dev_slot >= static_cast<int>(h->dev.size())) return fail(LDPCB200_EINVAL, "bad handle / dev_slot");
+    DeviceCtx *d;
+    cudaStream_t st;
+    int rc = device_of(h, dev_slot, stream, d, st);
+    if (rc) return rc;
     if (B <= 0) return 0;
     if (!d_true_err_words || !d_err_words || !d_syn_words || !d_out) return fail(LDPCB200_EINVAL, "null device buffer");
-    DeviceCtx &d = h->dev[dev_slot];
-    CU(cudaSetDevice(d.device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d.stream;
-    int rc = d.scratch.reserve(static_cast<size_t>(B) * h->SW * 4);
-    if (rc) return rc;
-    bp::score_rows_logical<<<grid_for(B * 32, d.sm_count), 256, 0, st>>>(d.d_colptr, d.d_ve_chk, h->NW, h->SW, B, d_true_err_words, d_err_words,
-                                                                        d_syn_words, d.scratch.as<uint32_t>(),
-                                                                        h->lmask.empty() ? nullptr : d.lmask.as<unsigned long long>(), d_out);
+    CU(cudaSetDevice(d->device));
+    if ((rc = d->scratch.reserve(static_cast<size_t>(B) * h->SW * 4))) return rc;
+    bp::score_rows_logical<<<grid_for(B * 32, d->sm_count), 256, 0, st>>>(d->d_colptr, d->d_ve_chk, h->NW, h->SW, B, d_true_err_words, d_err_words,
+                                                                         d_syn_words, d->scratch.as<uint32_t>(),
+                                                                         h->lmask.empty() ? nullptr : d->lmask.as<unsigned long long>(), d_out);
     h->launches++;
     CU(cudaGetLastError());
     return 0;
@@ -2106,17 +2026,7 @@ int ldpcb200_set_per(ldpcb200_t *h, double per)
     if (!h) return fail(LDPCB200_EINVAL, "null handle");
     if (h->variant != LDPCB200_VARIANT_EXACT && !(per > 0.0 && per < 1.0))
         return fail(LDPCB200_EINVAL, "the log-likelihood-ratio variants need 0 < per < 1 (finite prior)");
-    volatile double one_minus = 1.0 - per;
-    volatile double q = per / one_minus;
-    h->per = per;
-    for (DeviceCtx &d : h->dev) d.f_ready = false;        // the first-iteration tables depend on the prior
-    h->p0 = q;
-    h->regular_p0 = std::isnormal(h->p0) && h->p0 > 0.0;
-    if (h->variant != LDPCB200_VARIANT_EXACT) {
-        volatile double r = one_minus / per;
-        h->p0 = std::log(r);
-        if (h->variant == LDPCB200_VARIANT_FAST32) h->p0 = static_cast<double>(static_cast<float>(h->p0));
-    }
+    set_prior(h, per);
     return 0;
 }
 
@@ -2131,39 +2041,17 @@ static int sample_score_impl(ldpcb200_t *h, int64_t shots, int64_t first, uint64
     int rc = configure(h);
     if (rc) return rc;
     const int nd = static_cast<int>(h->dev.size());
-    std::vector<int64_t> lo(nd + 1, 0);
-    const int64_t blocks = (shots + 31) / 32;
-    for (int k = 0; k <= nd; ++k) lo[k] = std::min<int64_t>(shots, (blocks * k / nd) * 32);
-    lo[nd] = shots;
-    std::vector<int> rcs(nd, 0);
-    std::vector<std::string> errs(nd);
     std::vector<int64_t> ctr(static_cast<size_t>(nd) * LDPCB200_NUM_HARNESS_COUNTERS, 0);
-    auto work = [&](int k) {
-        rcs[k] = harness_on_device(h, h->dev[k], first + lo[k], lo[k + 1] - lo[k], seed, per_channel, osd != 0, ots,
-                                   &ctr[static_cast<size_t>(k) * LDPCB200_NUM_HARNESS_COUNTERS]);
-        if (rcs[k]) errs[k] = g_err;
-    };
-    if (nd == 1) {
-        work(0);
-    } else {
-        std::vector<std::thread> th;
-        for (int k = 0; k < nd; ++k) th.emplace_back(work, k);
-        for (auto &t : th) t.join();
-    }
-    for (int k = 0; k < nd; ++k)
-        if (rcs[k]) { g_err = errs[k]; return rcs[k]; }
-    bool summed = false;
-    if (nd > 1) {
-        nccl_prepare(h);
-        if (h->nccl_state == 1) {                          // one grouped ncclAllReduce of the 8 counters (K7 of SURVEY section 2)
-            rc = nccl_sum_block(h, LDPCB200_NUM_HARNESS_COUNTERS, [](DeviceCtx &d) { return d.hs_ctr.p; }, out);
-            if (rc) return rc;
-            summed = true;
-        }
-    }
-    if (!summed)
-        for (int k = 0; k < nd; ++k)
-            for (int c = 0; c < LDPCB200_NUM_HARNESS_COUNTERS; ++c) out[c] += ctr[static_cast<size_t>(k) * LDPCB200_NUM_HARNESS_COUNTERS + c];
+    // every device runs, even with no shots: that zeroes its counter block for the sum below
+    rc = fan_out(h, shots, [&](int k, int64_t s0, int64_t count) {
+        return harness_on_device(h, h->dev[k], first + s0, count, seed, per_channel, osd != 0, ots,
+                                 &ctr[static_cast<size_t>(k) * LDPCB200_NUM_HARNESS_COUNTERS]);
+    });
+    if (rc) return rc;
+    if (nd > 1) nccl_prepare(h);
+    if (h->nccl_state == 1)                                // one grouped ncclAllReduce of the 8 counters (K7 of SURVEY section 2)
+        return nccl_sum_block(h, LDPCB200_NUM_HARNESS_COUNTERS, [](DeviceCtx &d) { return d.hs_ctr.p; }, out);
+    host_sum(ctr, LDPCB200_NUM_HARNESS_COUNTERS, out);
     return 0;
 }
 
@@ -2198,14 +2086,17 @@ int ldpcb200_selftest_division(int32_t device, int32_t mode, uint64_t n, uint64_
 
 int ldpcb200_kernel_profile(ldpcb200_t *h, int32_t dev_slot, int64_t *out8, int32_t reset)
 {
-    if (!h || !out8 || dev_slot < 0 || dev_slot >= static_cast<int>(h->dev.size())) return fail(LDPCB200_EINVAL, "bad argument");
-    DeviceCtx &d = h->dev[dev_slot];
-    CU(cudaSetDevice(d.device));
+    DeviceCtx *d;
+    cudaStream_t st;
+    int rc = device_of(h, dev_slot, nullptr, d, st);
+    if (rc) return rc;
+    if (!out8) return fail(LDPCB200_EINVAL, "out8 is null");
+    CU(cudaSetDevice(d->device));
     CU(cudaDeviceSynchronize());
     unsigned long long v[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    if (d.kprof.p) {
-        CU(cudaMemcpy(v, d.kprof.p, 64, cudaMemcpyDeviceToHost));
-        if (reset) CU(cudaMemset(d.kprof.p, 0, 64));
+    if (d->kprof.p) {
+        CU(cudaMemcpy(v, d->kprof.p, 64, cudaMemcpyDeviceToHost));
+        if (reset) CU(cudaMemset(d->kprof.p, 0, 64));
     }
     for (int k = 0; k < 8; ++k) out8[k] = static_cast<int64_t>(v[k]);
     return 0;
@@ -2213,21 +2104,24 @@ int ldpcb200_kernel_profile(ldpcb200_t *h, int32_t dev_slot, int64_t *out8, int3
 
 int ldpcb200_kernel_time(ldpcb200_t *h, int32_t dev_slot, double *ms, int64_t *launches, int32_t reset)
 {
-    if (!h || !ms || !launches || dev_slot < 0 || dev_slot >= static_cast<int>(h->dev.size())) return fail(LDPCB200_EINVAL, "bad argument");
-    DeviceCtx &d = h->dev[dev_slot];
-    CU(cudaSetDevice(d.device));
+    DeviceCtx *d;
+    cudaStream_t st;
+    int rc = device_of(h, dev_slot, nullptr, d, st);
+    if (rc) return rc;
+    if (!ms || !launches) return fail(LDPCB200_EINVAL, "null argument");
+    CU(cudaSetDevice(d->device));
     CU(cudaDeviceSynchronize());
-    for (auto &pr : d.ktime_events) {
+    for (auto &pr : d->ktime_events) {
         float t = 0.f;
-        if (cudaEventElapsedTime(&t, pr.first, pr.second) == cudaSuccess) { d.ktime_ms += t; d.ktime_launches++; }
+        if (cudaEventElapsedTime(&t, pr.first, pr.second) == cudaSuccess) { d->ktime_ms += t; d->ktime_launches++; }
         else cudaGetLastError();
         cudaEventDestroy(pr.first);
         cudaEventDestroy(pr.second);
     }
-    d.ktime_events.clear();
-    *ms = d.ktime_ms;
-    *launches = d.ktime_launches;
-    if (reset) { d.ktime_ms = 0.0; d.ktime_launches = 0; }
+    d->ktime_events.clear();
+    *ms = d->ktime_ms;
+    *launches = d->ktime_launches;
+    if (reset) { d->ktime_ms = 0.0; d->ktime_launches = 0; }
     return 0;
 }
 
