@@ -16,7 +16,7 @@ SOURCES = (["ldpcb200.cu"] + ["bp_inst_m%d_b%d.cu" % (m, b) for m in (0, 1, 2) f
            + ["bp_inst_m%d_b0_minsum.cu" % m for m in (0, 1, 2)] + ["bp_inst_m%d_b0_fast.cu" % m for m in (0, 1, 2)] + ["bp_inst_single.cu", "bp_inst_single_minsum.cu", "bp_inst_smem.cu", "bp_inst_smem_minsum.cu",
               "bp_inst_single_fast.cu", "bp_inst_smem_fast.cu"])
 KERNEL_HEADERS = ["bp_math.cuh", "bp_kernel.cuh", "bp_smem.cuh", "bp_smem_inst.cuh", "bp_launch.h", "bp_launch_inst.cuh",
-                  "bp_filter.cuh", "bp_single.h", "bp_single.cuh", "../../include/ldpcb200.h"]
+                  "bp_filter.cuh", "bp_single.h", "bp_single.cuh", "bp_single_inst.cuh", "../../include/ldpcb200.h"]
 HEADERS = KERNEL_HEADERS + ["formats.cuh", "osd.cuh", "bpots.cuh"]
 
 NVCC_FLAGS = [

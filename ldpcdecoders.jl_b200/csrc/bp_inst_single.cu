@@ -1,29 +1,2 @@
-// the node-parallel small-batch kernel (exact variant) in its own translation unit
 #define BP_VARIANT 0
-#include "bp_single.cuh"
-
-namespace bp {
-
-cudaError_t single_launch_0(int grid, int smem_bytes, cudaStream_t st, const SingleParams &p)
-{
-    auto k = bp_node_parallel_kernel<kSingleThreads>;
-    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
-    if (e != cudaSuccess) return e;
-    k<<<grid, kSingleThreads, smem_bytes, st>>>(p);
-    return cudaGetLastError();
-}
-
-cudaError_t grid_kernel_occupancy_0(int *blocks_per_sm)
-{
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, bp_grid_kernel<kGridThreads>, kGridThreads, 0);
-}
-
-cudaError_t grid_launch_0(int grid, cudaStream_t st, const GridParams &p)
-{
-    // cooperative launch: the runtime guarantees that all CTAs are co-resident (the kernel spins on a grid-wide barrier)
-    GridParams q = p;
-    void *args[] = {&q};
-    return cudaLaunchCooperativeKernel(reinterpret_cast<const void *>(bp_grid_kernel<kGridThreads>), dim3(grid), dim3(kGridThreads), args, 0, st);
-}
-
-}  // namespace bp
+#include "bp_single_inst.cuh"

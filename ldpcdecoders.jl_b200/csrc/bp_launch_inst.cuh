@@ -1,5 +1,6 @@
 // bp_launch_inst.cuh -- body of one (BP_INST_MODE, BP_INST_BIG, BP_VARIANT) translation unit.
 #include "bp_launch.h"
+#include "bp_kernel.cuh"
 
 #define BP_CAT4(a, b, c, d) a##b##_##c##_##d
 #define BP_NAME4(prefix, m, b, v) BP_CAT4(prefix, m, b, v)
@@ -8,57 +9,26 @@
 namespace bp {
 
 template <int MAXT, int MINB>
-static cudaError_t attrs_one(int smem_bytes, int threads, int *blocks_per_sm)
-{
-    auto k = bp_persistent_kernel<BP_INST_MODE, BP_INST_BIG != 0, MAXT, MINB>;
-    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
-    if (e != cudaSuccess) return e;
-    if (BP_INST_MODE == 0) {
-        e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-        if (e != cudaSuccess) return e;
-    }
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, k, threads, smem_bytes);
-}
+static const void *entry() { return reinterpret_cast<const void *>(bp_persistent_kernel<BP_INST_MODE, BP_INST_BIG != 0, MAXT, MINB>); }
 
-cudaError_t BP_NAME(kernel_attrs_, BP_INST_MODE, BP_INST_BIG)(int shape, int smem_bytes, int threads, int *bps)
-{
-    if (shape == kShape256x2) return attrs_one<256, 2>(smem_bytes, threads, bps);
+// (the #if blocks keep the absent shapes from being instantiated at all)
+const void *const BP_NAME(persistent_kernels_, BP_INST_MODE, BP_INST_BIG)[kShapes] = {
+    entry<256, 2>(),
 #if !BP_INST_BIG
-    if (shape == kShape384x2) return attrs_one<384, 2>(smem_bytes, threads, bps);
-#endif
-#if !BP_INST_BIG && BP_INST_MODE >= 1
-    if (shape == kShape320x2) return attrs_one<320, 2>(smem_bytes, threads, bps);
+    entry<384, 2>(),
+#else
+    nullptr,
 #endif
 #if BP_INST_MODE == 0
-    if (shape == kShape512x1) return attrs_one<512, 1>(smem_bytes, threads, bps);
-#endif
-    return cudaErrorInvalidConfiguration;
-}
-
-// The dynamic-shared-memory limit is an attribute of the kernel instantiation on the current device, not of a
-// decoder handle: two live handles that share an instantiation but need different sizes would otherwise lower
-// each other's limit.  It is therefore (re)set before every launch (a host-side call of about a microsecond).
-template <int MAXT, int MINB>
-static void launch_one(int grid, int threads, int smem_bytes, cudaStream_t st, const KernelParams &p)
-{
-    auto k = bp_persistent_kernel<BP_INST_MODE, BP_INST_BIG != 0, MAXT, MINB>;
-    if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes) != cudaSuccess) return;   // surfaces through cudaGetLastError
-    k<<<grid, threads, smem_bytes, st>>>(p);
-}
-
-void BP_NAME(kernel_launch_, BP_INST_MODE, BP_INST_BIG)(int shape, int grid, int threads, int smem_bytes, cudaStream_t st,
-                                                        const KernelParams &p)
-{
-    if (shape == kShape256x2) launch_one<256, 2>(grid, threads, smem_bytes, st, p);
-#if !BP_INST_BIG
-    if (shape == kShape384x2) launch_one<384, 2>(grid, threads, smem_bytes, st, p);
+    entry<512, 1>(),
+#else
+    nullptr,
 #endif
 #if !BP_INST_BIG && BP_INST_MODE >= 1
-    if (shape == kShape320x2) launch_one<320, 2>(grid, threads, smem_bytes, st, p);
+    entry<320, 2>(),
+#else
+    nullptr,
 #endif
-#if BP_INST_MODE == 0
-    if (shape == kShape512x1) launch_one<512, 1>(grid, threads, smem_bytes, st, p);
-#endif
-}
+};
 
 }  // namespace bp

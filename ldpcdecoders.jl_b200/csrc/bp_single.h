@@ -38,17 +38,13 @@ struct GridParams {
     unsigned int *bar;      // [2] barrier counters (zero on entry and on exit)
 };
 constexpr int kGridThreads = 256;
-// max co-resident CTAs per SM of the grid kernel (0 on error); launch with exactly grid CTAs <= that x SMs
-cudaError_t grid_kernel_occupancy_0(int *blocks_per_sm);
-cudaError_t grid_kernel_occupancy_1(int *blocks_per_sm);
-cudaError_t grid_kernel_occupancy_2(int *blocks_per_sm);
-cudaError_t grid_launch_0(int grid, cudaStream_t st, const GridParams &p);
-cudaError_t grid_launch_1(int grid, cudaStream_t st, const GridParams &p);
-cudaError_t grid_launch_2(int grid, cudaStream_t st, const GridParams &p);
-
 constexpr int kSingleThreads = 512;
-cudaError_t single_launch_0(int grid, int smem_bytes, cudaStream_t st, const SingleParams &p);   // exact variant
-cudaError_t single_launch_1(int grid, int smem_bytes, cudaStream_t st, const SingleParams &p);   // min-sum variant
-cudaError_t single_launch_2(int grid, int smem_bytes, cudaStream_t st, const SingleParams &p);   // fast FP32 variant
+
+// Entry points of one variant's bp_node_parallel_kernel<kSingleThreads> and bp_grid_kernel<kGridThreads>
+// (bp_single_inst.cuh).  The grid kernel needs a cooperative launch with no more CTAs than can be co-resident.
+struct SingleKernels {
+    const void *node_parallel, *grid;
+};
+extern const SingleKernels single_kernels_0, single_kernels_1, single_kernels_2;   // exact, min-sum, fast FP32 variant
 
 }  // namespace bp

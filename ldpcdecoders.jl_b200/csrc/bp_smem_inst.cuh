@@ -9,47 +9,17 @@
 
 namespace bp {
 
-template <int MAXT, int MINB, bool EB64>
-static cudaError_t smem_attrs_one(int smem_bytes, int threads, int *blocks_per_sm)
-{
-    auto k = bp_smem_kernel<MAXT, MINB, EB64>;
-    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    if (e != cudaSuccess) return e;
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, k, threads, smem_bytes);
-}
+template <int MAXT, int MINB, bool EB64, bool PROF = false, bool DUAL = false>
+static const void *entry() { return reinterpret_cast<const void *>(bp_smem_kernel<MAXT, MINB, EB64, PROF, DUAL>); }
 
-cudaError_t BPS_NAME(smem_kernel_attrs_)(int shape, int eb64, int smem_bytes, int threads, int *bps)
-{
-    if (shape == kShape256x2) return eb64 ? smem_attrs_one<256, 2, true>(smem_bytes, threads, bps) : smem_attrs_one<256, 2, false>(smem_bytes, threads, bps);
-    if (shape == kShape384x2) return eb64 ? smem_attrs_one<384, 2, true>(smem_bytes, threads, bps) : smem_attrs_one<384, 2, false>(smem_bytes, threads, bps);
-    if (shape == kShape512x1) return eb64 ? smem_attrs_one<512, 1, true>(smem_bytes, threads, bps) : smem_attrs_one<512, 1, false>(smem_bytes, threads, bps);
-    return cudaErrorInvalidConfiguration;
-}
-
-// the shared-memory limit is (re)set before every launch: it belongs to the instantiation, not to a handle
-template <int MAXT, int MINB, bool EB64>
-static void smem_launch_one(int grid, int threads, int smem_bytes, cudaStream_t st, const KernelParams &p)
-{
-    auto k = bp_smem_kernel<MAXT, MINB, EB64>;
-    if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes) != cudaSuccess) return;
-    k<<<grid, threads, smem_bytes, st>>>(p);
-}
-
-void BPS_NAME(smem_kernel_launch_)(int shape, int eb64, int grid, int threads, int smem_bytes, cudaStream_t st, const KernelParams &p)
-{
-    if (shape == kShape256x2 && !eb64 && p.prof != nullptr) {      // phase-timing build (diagnostics)
-        auto k = bp_smem_kernel<256, 2, false, true>;
-        if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes) != cudaSuccess) return;
-        k<<<grid, threads, smem_bytes, st>>>(p);
-        return;
-    }
-    if (shape == kShape256x2) { if (eb64) smem_launch_one<256, 2, true>(grid, threads, smem_bytes, st, p); else smem_launch_one<256, 2, false>(grid, threads, smem_bytes, st, p); }
-    if (shape == kShape384x2) { if (eb64) smem_launch_one<384, 2, true>(grid, threads, smem_bytes, st, p); else smem_launch_one<384, 2, false>(grid, threads, smem_bytes, st, p); }
-    if (shape == kShape512x1) { if (eb64) smem_launch_one<512, 1, true>(grid, threads, smem_bytes, st, p); else smem_launch_one<512, 1, false>(grid, threads, smem_bytes, st, p); }
-}
-
+const SmemKernels BPS_NAME(smem_kernels_) = {
+    {{entry<256, 2, false>(), entry<256, 2, true>()},
+     {entry<384, 2, false>(), entry<384, 2, true>()},
+     {entry<512, 1, false>(), entry<512, 1, true>()},
+     {nullptr, nullptr},                                                          // kShape320x2: HBM modes only
+     {entry<512, 1, false, false, true>(), entry<512, 1, true, false, true>()}},  // kSmemDual
+    {entry<256, 2, false, true>(), nullptr, nullptr, nullptr, entry<512, 1, false, true, true>()},
+};
 
 // ---- tables of the first-iteration filter, computed with this variant's node updates (bp_filter.cuh)
 cudaError_t BPS_NAME(filter_setup_)(const FilterSetup &q, cudaStream_t st)
@@ -57,30 +27,6 @@ cudaError_t BPS_NAME(filter_setup_)(const FilterSetup &q, cudaStream_t st)
     first_iter_check_table_kernel<<<1, 32, 0, st>>>(q);
     first_iter_truth_table_kernel<<<(q.n + 127) / 128, 128, 0, st>>>(q);
     return cudaGetLastError();
-}
-
-// ---- dual-team form: one CTA of 2 x W warps per SM (bp_smem_kernel<512, 1, EB64, PROF, true>)
-cudaError_t BPS_NAME(smem_dual_attrs_)(int eb64, int smem_bytes, int threads, int *bps)
-{
-    auto set = [&](auto k) -> cudaError_t {
-        cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-        if (e != cudaSuccess) return e;
-        return cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, k, threads, smem_bytes);
-    };
-    return eb64 ? set(bp_smem_kernel<512, 1, true, false, true>) : set(bp_smem_kernel<512, 1, false, false, true>);
-}
-
-void BPS_NAME(smem_dual_launch_)(int eb64, int grid, int threads, int smem_bytes, cudaStream_t st, const KernelParams &p)
-{
-    auto go = [&](auto k) {
-        if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes) != cudaSuccess) return;
-        k<<<grid, threads, smem_bytes, st>>>(p);
-    };
-    if (!eb64 && p.prof != nullptr) go(bp_smem_kernel<512, 1, false, true, true>);      // phase-timing build (diagnostics)
-    else if (eb64) go(bp_smem_kernel<512, 1, true, false, true>);
-    else go(bp_smem_kernel<512, 1, false, false, true>);
 }
 
 }  // namespace bp

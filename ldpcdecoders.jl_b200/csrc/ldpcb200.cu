@@ -22,8 +22,8 @@
 #include "../../include/ldpcb200.h"
 #define BP_WITH_SELFTEST 1
 #define BP_FILTER_KERNEL 1
+#include "bp_kernel.cuh"
 #include "bp_launch.h"
-#include "bp_math.cuh"
 #include "bp_single.h"
 #include "formats.cuh"
 #include "osd.cuh"
@@ -229,6 +229,8 @@ struct ldpcb200 {
     bool lean = false, eb64 = false;   // bp_smem_kernel selected / its decision fields are 64 bits wide
     bool dual = false;                 // ... in its two-teams-per-CTA form
     int opt_dual = 0;                  // (measured equal to two independent CTAs per SM on C3: kept as an option, see DESIGN.md)
+    const void *kernel = nullptr;      // entry point of the batch kernel configure() selected ...
+    const void *kernel_prof = nullptr; // ... and the one that runs with option kernel_profile (its phase-timing build, if any)
     bp::KernelParams kp_proto{};
     std::vector<DeviceCtx> dev;
     std::atomic<long long> launches{0};
@@ -598,38 +600,52 @@ int kernel_shape(bool two_ctas, int threads, int mode = 0, bool big = false)
 }
 
 // The compiled kernels of one variant.  The instantiations live in their own translation units (bp_inst_*.cu); the
-// persistent kernel's are indexed [mode][big], nullptr where none exists (the min-sum and fast variants have no
-// local-memory degree path: ldpcb200_create refuses those codes).
+// persistent kernel's are indexed [mode][big][shape], nullptr where none exists (the min-sum and fast variants have
+// no local-memory degree path: ldpcb200_create refuses those codes).
 struct VariantKernels {
-    decltype(&bp::kernel_attrs_0_0_0) attrs[3][2];
-    decltype(&bp::kernel_launch_0_0_0) launch[3][2];
-    decltype(&bp::smem_kernel_attrs_0) smem_attrs;
-    decltype(&bp::smem_kernel_launch_0) smem_launch;
-    decltype(&bp::smem_dual_attrs_0) dual_attrs;
-    decltype(&bp::smem_dual_launch_0) dual_launch;
-    decltype(&bp::filter_setup_0) filter_setup;
-    decltype(&bp::grid_kernel_occupancy_0) grid_occupancy;
-    decltype(&bp::grid_launch_0) grid_launch;
-    decltype(&bp::single_launch_0) single_launch;
+    const void *const *persistent[3][2];
+    const bp::SmemKernels *smem;
+    cudaError_t (*filter_setup)(const bp::FilterSetup &, cudaStream_t);
+    const bp::SingleKernels *single;
 };
 
 const VariantKernels kVariantKernels[3] = {
-    {{{bp::kernel_attrs_0_0_0, bp::kernel_attrs_0_1_0}, {bp::kernel_attrs_1_0_0, bp::kernel_attrs_1_1_0}, {bp::kernel_attrs_2_0_0, bp::kernel_attrs_2_1_0}},
-     {{bp::kernel_launch_0_0_0, bp::kernel_launch_0_1_0}, {bp::kernel_launch_1_0_0, bp::kernel_launch_1_1_0}, {bp::kernel_launch_2_0_0, bp::kernel_launch_2_1_0}},
-     bp::smem_kernel_attrs_0, bp::smem_kernel_launch_0, bp::smem_dual_attrs_0, bp::smem_dual_launch_0, bp::filter_setup_0,
-     bp::grid_kernel_occupancy_0, bp::grid_launch_0, bp::single_launch_0},
-    {{{bp::kernel_attrs_0_0_1, nullptr}, {bp::kernel_attrs_1_0_1, nullptr}, {bp::kernel_attrs_2_0_1, nullptr}},
-     {{bp::kernel_launch_0_0_1, nullptr}, {bp::kernel_launch_1_0_1, nullptr}, {bp::kernel_launch_2_0_1, nullptr}},
-     bp::smem_kernel_attrs_1, bp::smem_kernel_launch_1, bp::smem_dual_attrs_1, bp::smem_dual_launch_1, bp::filter_setup_1,
-     bp::grid_kernel_occupancy_1, bp::grid_launch_1, bp::single_launch_1},
-    {{{bp::kernel_attrs_0_0_2, nullptr}, {bp::kernel_attrs_1_0_2, nullptr}, {bp::kernel_attrs_2_0_2, nullptr}},
-     {{bp::kernel_launch_0_0_2, nullptr}, {bp::kernel_launch_1_0_2, nullptr}, {bp::kernel_launch_2_0_2, nullptr}},
-     bp::smem_kernel_attrs_2, bp::smem_kernel_launch_2, bp::smem_dual_attrs_2, bp::smem_dual_launch_2, bp::filter_setup_2,
-     bp::grid_kernel_occupancy_2, bp::grid_launch_2, bp::single_launch_2},
+    {{{bp::persistent_kernels_0_0_0, bp::persistent_kernels_0_1_0}, {bp::persistent_kernels_1_0_0, bp::persistent_kernels_1_1_0},
+      {bp::persistent_kernels_2_0_0, bp::persistent_kernels_2_1_0}},
+     &bp::smem_kernels_0, bp::filter_setup_0, &bp::single_kernels_0},
+    {{{bp::persistent_kernels_0_0_1, nullptr}, {bp::persistent_kernels_1_0_1, nullptr}, {bp::persistent_kernels_2_0_1, nullptr}},
+     &bp::smem_kernels_1, bp::filter_setup_1, &bp::single_kernels_1},
+    {{{bp::persistent_kernels_0_0_2, nullptr}, {bp::persistent_kernels_1_0_2, nullptr}, {bp::persistent_kernels_2_0_2, nullptr}},
+     &bp::smem_kernels_2, bp::filter_setup_2, &bp::single_kernels_2},
 };
 
 // (indexed by LDPCB200_VARIANT_*, which ldpcb200_create checks)
 const VariantKernels &kernels_of(int variant) { return kVariantKernels[variant]; }
+
+// Shared-memory limit (and, where the messages live in shared memory, the carveout) of a kernel instantiation on the
+// current device, then how many of its CTAs an SM holds.  A nullptr entry is no instantiation: configure never picks one.
+cudaError_t kernel_attrs(const void *k, bool carveout, int smem_bytes, int threads, int *blocks_per_sm)
+{
+    if (!k) return cudaErrorInvalidDeviceFunction;
+    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
+    if (e == cudaSuccess && carveout)
+        e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, k, threads, smem_bytes);
+    return e;
+}
+
+// The dynamic-shared-memory limit is an attribute of the kernel instantiation on the current device, not of a decoder
+// handle: two live handles that share an instantiation but need different sizes would otherwise lower each other's
+// limit.  It is therefore (re)set before every launch (a host-side call of about a microsecond).
+template <class P>
+cudaError_t launch_kernel(const void *k, int grid, int threads, int smem_bytes, cudaStream_t st, const P &p)
+{
+    if (!k) return cudaErrorInvalidDeviceFunction;
+    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
+    if (e != cudaSuccess) return e;
+    void *args[] = {const_cast<P *>(&p)};
+    return cudaLaunchKernel(k, dim3(grid), dim3(threads), args, smem_bytes, st);
+}
 
 // Warps per CTA: warp w owns checks w, w+W, ... and variables w, w+W, ...; pick the W whose two
 // round-robin splits waste the fewest warp-slots (ties -> more warps, better latency hiding).
@@ -770,22 +786,23 @@ int configure(ldpcb200 *h)
         CU(cudaSetDevice(d0.device));
     }
     const VariantKernels &K = kernels_of(h->variant);
+    const int form = dual ? bp::kSmemDual : shape;
+    const void *const *persistent = K.persistent[mode][h->big];
+    const void *kernel = lean ? K.smem->kernel[form][eb64] : persistent ? persistent[shape] : nullptr;
     int bps = 0;
     for (DeviceCtx &d : h->dev) {
         CU(cudaSetDevice(d.device));
-        if (lean) {
-            cudaError_t e = dual ? K.dual_attrs(eb64, need, 2 * warps * 32, &bps) : K.smem_attrs(shape, eb64, need, warps * 32, &bps);
-            if (e != cudaSuccess) return fail(LDPCB200_ECUDA, "kernel attributes (shared-memory kernel): %s", cudaGetErrorString(e));
-        } else {
-            cudaError_t e = K.attrs[mode][h->big](shape, need, warps * 32, &bps);
-            if (e != cudaSuccess) return fail(LDPCB200_ECUDA, "kernel attributes (mode %d): %s", mode, cudaGetErrorString(e));
-        }
+        const cudaError_t e = kernel_attrs(kernel, mode == 0, need, (dual ? 2 : 1) * warps * 32, &bps);
+        if (e != cudaSuccess && lean) return fail(LDPCB200_ECUDA, "kernel attributes (shared-memory kernel): %s", cudaGetErrorString(e));
+        if (e != cudaSuccess) return fail(LDPCB200_ECUDA, "kernel attributes (mode %d): %s", mode, cudaGetErrorString(e));
     }
     if (bps < 1) return fail(LDPCB200_EUNSUPPORTED, "BP kernel (mode %d, %d threads, %d B smem) does not fit on an SM", mode, warps * 32, need);
     if (h->opt_max_ctas > 0) bps = std::min(bps, h->opt_max_ctas);
     h->family = family; h->mode = mode; h->warps = warps; h->shape = shape; h->ctas_per_sm = bps;
     h->smem_bytes = need; h->nfw = nfw; h->efield_global = ef_global; h->kp_proto = kp;
     h->lean = lean; h->eb64 = eb64; h->dual = dual;
+    h->kernel = kernel;
+    h->kernel_prof = lean && !eb64 && K.smem->prof[form] ? K.smem->prof[form] : kernel;
     h->slots = (dual ? 64 : 32) * bps * d0.sm_count;
     h->configured = true;
     return 0;
@@ -896,7 +913,7 @@ int decode_on_device(ldpcb200 *h, DeviceCtx &d, int64_t B, const uint32_t *syn_w
             if (d.gk_blocks_per_sm < 0) {
                 int coop = 0, bps = 0;
                 cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, d.device);
-                cudaError_t e = K.grid_occupancy(&bps);
+                cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, K.single->grid, bp::kGridThreads, 0);
                 if (e != cudaSuccess) { cudaGetLastError(); bps = 0; }
                 d.gk_blocks_per_sm = coop ? bps : 0;
             }
@@ -915,7 +932,9 @@ int decode_on_device(ldpcb200 *h, DeviceCtx &d, int64_t B, const uint32_t *syn_w
                 q.msg = d.gk_msg.as<double>();
                 q.resid = d.gk_state.as<uint32_t>(); q.dec = q.resid + h->SW;
                 q.work = reinterpret_cast<int *>(q.dec + h->NW); q.bar = reinterpret_cast<unsigned int *>(q.work + 2);
-                CU(K.grid_launch(grid, st, q));
+                // cooperative launch: the runtime guarantees that all CTAs are co-resident (the kernel spins on a grid-wide barrier)
+                void *args[] = {&q};
+                CU(cudaLaunchCooperativeKernel(K.single->grid, dim3(grid), dim3(bp::kGridThreads), args, 0, st));
                 h->launches++;
                 return 0;
             }
@@ -924,7 +943,7 @@ int decode_on_device(ldpcb200 *h, DeviceCtx &d, int64_t B, const uint32_t *syn_w
             bp::SingleParams q{};
             common(q);
             q.off_syn = off_syn; q.off_resid = off_syn + h->SW * 4; q.off_dec = off_syn + 2 * h->SW * 4;
-            CU(K.single_launch(static_cast<int>(B), smem, st, q));
+            CU(launch_kernel(K.single->node_parallel, static_cast<int>(B), bp::kSingleThreads, smem, st, q));
             h->launches++;
             return 0;
         }
@@ -1014,13 +1033,9 @@ int decode_on_device(ldpcb200 *h, DeviceCtx &d, int64_t B, const uint32_t *syn_w
             }
             const long long groups = (Bl + 31) / 32;
             KernelTimer timer(h, d, st);
-            if (h->dual) {
-                const int gl = static_cast<int>(std::min<long long>((groups + 1) / 2, static_cast<long long>(d.sm_count) * h->ctas_per_sm));
-                K.dual_launch(h->eb64, gl, 2 * thr, h->smem_bytes, st, q);
-            } else {
-                const int gl = static_cast<int>(std::min<long long>(groups, static_cast<long long>(d.sm_count) * h->ctas_per_sm));
-                K.smem_launch(h->shape, h->eb64, gl, thr, h->smem_bytes, st, q);
-            }
+            const int teams = h->dual ? 2 : 1;
+            const int gl = static_cast<int>(std::min<long long>((groups + teams - 1) / teams, static_cast<long long>(d.sm_count) * h->ctas_per_sm));
+            CU(launch_kernel(q.prof ? h->kernel_prof : h->kernel, gl, teams * thr, h->smem_bytes, st, q));
             h->launches++;
         }
     } else {
@@ -1030,7 +1045,7 @@ int decode_on_device(ldpcb200 *h, DeviceCtx &d, int64_t B, const uint32_t *syn_w
             p.queue_ctr = f_count.as<unsigned int>() + 2;
         }
         KernelTimer timer(h, d, st);
-        K.launch[h->mode][h->big](h->shape, grid, thr, h->smem_bytes, st, p);
+        CU(launch_kernel(h->kernel, grid, thr, h->smem_bytes, st, p));
         h->launches++;
     }
     CU(cudaGetLastError());

@@ -17,7 +17,6 @@
 // One CTA per syndrome (work queue over the unconverged list).  Shared memory holds the whole augmented
 // matrix bit-packed by rows over the SORTED column positions: m rows x NWr words, the last bit of a row is
 // its target bit; NWr is 4 x odd so that 16-byte row accesses of 8 consecutive rows are bank-conflict-free.
-// Stated deviation (as in the oracle): r = RN(1/R) instead of Julia's exp(log(1/R)).
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
@@ -59,6 +58,46 @@ __global__ void osd_fill_ones_kernel(double *p, long long nelem)
 
 constexpr int kOsdMaxRowsPerThread = 8;     // rows a thread owns: m <= 8 * T
 
+// Reliability keys of the columns (:53-54), padded to NP with the largest key: descending max(r, 1-r), ties by index
+// == ascending (~bits(max(r, 1-r)), index).  Stated deviation (as in the oracle): r = RN(1/R) instead of Julia's
+// exp(log(1/R)).
+template <int T>
+__device__ __forceinline__ void osd_keys(int tid, const double *R, int n, int NP, unsigned long long *key, int *idx)
+{
+    for (int j = tid; j < NP; j += T) {
+        unsigned long long kb = ~0ull;
+        if (j < n) {
+            const double r = __ddiv_rn(1.0, R[j]);
+            const double q = __dsub_rn(1.0, r);
+            kb = ~static_cast<unsigned long long>(__double_as_longlong(r > q ? r : q));
+        }
+        key[j] = kb;
+        idx[j] = j;
+    }
+}
+
+// Bitonic sort of the NP (key, idx) pairs into ascending order, which is the stable descending order of :55 (every
+// thread of the CTA calls it after a barrier that follows osd_keys; it ends with a barrier)
+template <int T>
+__device__ __forceinline__ void osd_sort(int tid, int NP, unsigned long long *key, int *idx)
+{
+    for (int k = 2; k <= NP; k <<= 1) {
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            for (int q = tid; q < NP / 2; q += T) {        // one compare-exchange per thread and trip, no idle lanes
+                const int i = ((q & ~(j - 1)) << 1) | (q & (j - 1)), x = i | j;
+                const unsigned long long ka = key[i], kb = key[x];
+                const int ia = idx[i], ib = idx[x];
+                const bool gt = ka > kb || (ka == kb && ia > ib);
+                if (gt == ((i & k) == 0)) {
+                    key[i] = kb; key[x] = ka;
+                    idx[i] = ib; idx[x] = ia;
+                }
+            }
+            __syncthreads();
+        }
+    }
+}
+
 template <int T, int RPT>                   // RPT = ceil(m / T)
 __global__ void __launch_bounds__(T, 1) osd0_kernel(const OsdParams p)
 {
@@ -94,37 +133,13 @@ __global__ void __launch_bounds__(T, 1) osd0_kernel(const OsdParams p)
         long long t0 = 0, c_sort = 0, c_build = 0, c_scan = 0, c_xor = 0, c_solve = 0;
         const bool prof = p.profile != 0 && tid == 0;
         if (prof) t0 = clock64();
-        // ---- reliability keys (:53-54): descending key, ties by index  ==  ascending (~bits(key), index)
-        for (int j = tid; j < NP; j += T) {
-            unsigned long long kb = ~0ull;
-            if (j < n) {
-                const double r = __ddiv_rn(1.0, R[j]);
-                const double q = __dsub_rn(1.0, r);
-                kb = ~static_cast<unsigned long long>(__double_as_longlong(r > q ? r : q));
-            }
-            key[j] = kb;
-            idx[j] = j;
-        }
+        // ---- reliability sort (:53-55)
+        osd_keys<T>(tid, R, n, NP, key, idx);
         for (int i = tid; i < m * (NWr / 4); i += T) reinterpret_cast<uint4 *>(Hs)[i] = make_uint4(0, 0, 0, 0);
         for (int r = tid; r < m; r += T) { piv[r] = -1; rowat[r] = r; }
         if (tid == 0) { ctl[2] = 0; ctl[12] = -1; }   // target count / solve round 0
         __syncthreads();
-        // bitonic sort of (key, idx) pairs
-        for (int k = 2; k <= NP; k <<= 1) {
-            for (int j = k >> 1; j > 0; j >>= 1) {
-                for (int q = tid; q < NP / 2; q += T) {        // one compare-exchange per thread and trip, no idle lanes
-                    const int i = ((q & ~(j - 1)) << 1) | (q & (j - 1)), x = i | j;
-                    const unsigned long long ka = key[i], kb = key[x];
-                    const int ia = idx[i], ib = idx[x];
-                    const bool gt = ka > kb || (ka == kb && ia > ib);
-                    if (gt == ((i & k) == 0)) {
-                        key[i] = kb; key[x] = ka;
-                        idx[i] = ib; idx[x] = ia;
-                    }
-                }
-                __syncthreads();
-            }
-        }
+        osd_sort<T>(tid, NP, key, idx);
         if (prof) { const long long t = clock64(); c_sort = t - t0; t0 = t; }
         // ---- H_sorted (:56) with the target column syndrome xor H*bp_err (:66-71) as the last bit of a row
         for (int r = tid; r < m; r += T)
@@ -337,36 +352,13 @@ __global__ void __launch_bounds__(T, 1) osdk_kernel(const OsdParams p, const int
         const double *R = p.ratio + b * n;
         uint32_t *erow = p.err_words + b * p.NW;
         const uint32_t *srow = p.syn_words + b * p.SW;
-        // ---- reliability keys and stable descending sort (:53-55), as osd0_kernel
-        for (int j = tid; j < NP; j += T) {
-            unsigned long long kb = ~0ull;
-            if (j < n) {
-                const double r = __ddiv_rn(1.0, R[j]);
-                const double q = __dsub_rn(1.0, r);
-                kb = ~static_cast<unsigned long long>(__double_as_longlong(r > q ? r : q));
-            }
-            key[j] = kb;
-            idx[j] = j;
-        }
+        // ---- reliability sort (:53-55)
+        osd_keys<T>(tid, R, n, NP, key, idx);
         for (int i = tid; i < m * (NWr / 4); i += T) reinterpret_cast<uint4 *>(Hs)[i] = make_uint4(0, 0, 0, 0);
         for (int r = tid; r < m; r += T) rowat[r] = r;
         for (int w = tid; w < NWr; w += T) ev[w] = 0u;
         __syncthreads();
-        for (int k = 2; k <= NP; k <<= 1) {
-            for (int j = k >> 1; j > 0; j >>= 1) {
-                for (int q = tid; q < NP / 2; q += T) {
-                    const int i = ((q & ~(j - 1)) << 1) | (q & (j - 1)), x = i | j;
-                    const unsigned long long ka = key[i], kb = key[x];
-                    const int ia = idx[i], ib = idx[x];
-                    const bool gt = ka > kb || (ka == kb && ia > ib);
-                    if (gt == ((i & k) == 0)) {
-                        key[i] = kb; key[x] = ka;
-                        idx[i] = ib; idx[x] = ia;
-                    }
-                }
-                __syncthreads();
-            }
-        }
+        osd_sort<T>(tid, NP, key, idx);
         // ---- [H_sorted | syndrome] (:56, :137) and bp_err over the sorted positions (:57)
         for (int r = tid; r < m; r += T)
             if ((srow[r >> 5] >> (r & 31)) & 1u) atomicOr(&Hs[r * NWr + augw], augm);
